@@ -4,6 +4,7 @@ with class-balanced thresholds.
 
   python bench.py --gpus N --steps K --warmup W              (N>1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W    (CPU reference arm, rank 0 only)
+  python bench.py ... --dump-outputs DIR                      (also write the last timed step's outputs as DIR/*.npy)
 
 Workload (BASELINE.json configs): N = 1 runs configs[1], 2,000 synthetic 480x256 images resident in HBM; N > 1 runs configs[2],
 a 20,000-image target set sharded by contiguous image range over the ranks (strong scaling: 10,000 / 5,000 / 2,500 images per
@@ -59,7 +60,14 @@ def parse_args():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--ref-images", type=int, default=32, help="--impl reference: images per step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy: rank 0 writes the global statistics "
+                         "and a seeded sample of its own shard's maps (see dump_outputs); --impl reference writes the "
+                         "class weights")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def images_total(args, world):
@@ -310,12 +318,15 @@ def run_reference(args):
             step()
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            step()
+            weights = step()
         el = time.perf_counter() - t0
     finally:
         if pool is not None:
             pool.shutdown()
         torch.set_num_threads(threads)
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "class_weights.npy"), weights.numpy().astype(np.float32))
     mpix = args.steps * n * args.height * args.width / 1e6
     val = round(mpix / el, 3)
     sample = ("%d synthetic %dx%d images x 3 sources per step (bounded sample of the workload), %s, %s.  Probe: %s"
@@ -443,6 +454,33 @@ def job_digest(job):
              job.final_hist.cpu().numpy().tobytes(), job.kept.cpu().numpy().tobytes(),
              np.int64(int(job.marginal)).tobytes()]
     return hashlib.sha256(b"".join(parts)).hexdigest()[:16]
+
+
+DUMP_SAMPLE_PIXELS = 1 << 21    # 4 maps x 8 MB + 16 MB of pixel index: well under 64 MB
+
+
+def dump_outputs(torch, job, out_dir, sample=DUMP_SAMPLE_PIXELS, seed=0):
+    """Write the LabelJob that LabelGenerator.run returned in the last timed step to out_dir/<name>.npy, so that two builds
+    can be compared output for output on the same seeded inputs.  The global thresholds and histograms are written in full;
+    the per-pixel maps of this rank's shard (2.2 GB at configs[1]) at a fixed, seeded sample of `sample` flat pixel positions,
+    stored beside them as `pixel_index`.  Maps and thresholds are float32, counts and the index float64 (exact).  A class that
+    is never kept (the ignore class) has threshold +inf; it is written as the largest float32, which no confidence in [0, 1]
+    reaches either, so that every dumped value is finite."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    npix = job.label.numel()
+    idx = np.sort(np.random.default_rng(seed).choice(npix, size=min(sample, npix), replace=False))
+    dev_idx = torch.from_numpy(idx).to(job.label.device)
+    thresh = job.thresh.cpu().numpy().astype(np.float32)
+    thresh[np.isposinf(thresh)] = np.finfo(np.float32).max
+    arrays = {"pixel_index": idx.astype(np.float64), "thresh": thresh,
+              "near_tie_pixels": np.array([int(job.marginal)], dtype=np.float64)}
+    for name in ("label", "final", "conf", "unc"):
+        arrays[name] = getattr(job, name).reshape(-1)[dev_idx].cpu().numpy().astype(np.float32)
+    for name in ("kept", "class_hist", "final_hist"):
+        arrays[name] = getattr(job, name).cpu().numpy().astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class Timer:
@@ -778,6 +816,8 @@ def main():
                "digest": job_digest(job),
                "digest_note": "sha256/16 of (thresholds, class_hist, final_hist, kept, near-tie count): identical for every rank "
                               "count on the same image set (compare configs[2] lines and secondary.configs2_one_gpu)"}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, job, args.dump_outputs)
     job = None
 
     # ---- end to end through the public host-buffer API -----------------------------------------------------------

@@ -47,11 +47,48 @@ def test_shard_plan_covers_the_named_configs():
     assert bench.shard_plan(a, 1) == (20000, 2500, 8)
 
 
-def test_reference_arm_prints_one_contract_line():
+def test_dump_outputs_writes_the_job_as_float_arrays(tmp_path):
+    """--dump-outputs: every array of the LabelJob as float32/float64 .npy, the maps at a seeded pixel sample that is the same
+    on every call, and the whole dump under 64 MB at the size of configs[1]."""
+    from mspl_b200.pipeline import LabelJob
+    n, h, w = 3, 16, 20
+    gen = torch.Generator().manual_seed(1)
+    label = torch.randint(0, 5, (n, h, w), generator=gen).to(torch.uint8)
+    final = torch.where(torch.rand(n, h, w, generator=gen) < 0.2, torch.full_like(label, 4), label)
+    conf, unc = torch.rand(n, h, w, generator=gen), torch.rand(n, h, w, generator=gen)
+    hist = torch.bincount(label.reshape(-1).long(), minlength=5)
+    job = LabelJob(label, final, None, conf, unc, torch.tensor([0.5, 0.25, 0.75, 0.125, float("inf")]), hist, hist,
+                   torch.bincount(final.reshape(-1).long(), minlength=5), torch.tensor(7))
+    for d in ("a", "b"):
+        bench.dump_outputs(torch, job, str(tmp_path / d), sample=100)
+    names = {"pixel_index", "label", "final", "conf", "unc", "thresh", "kept", "class_hist", "final_hist", "near_tie_pixels"}
+    assert {f[:-4] for f in os.listdir(tmp_path / "a")} == names
+    for name in names:
+        a, b = np.load(tmp_path / "a" / (name + ".npy")), np.load(tmp_path / "b" / (name + ".npy"))
+        assert a.dtype in (np.float32, np.float64) and np.isfinite(a).all() and np.array_equal(a, b), name
+    # the never-kept ignore class: +inf becomes the largest float32, the other thresholds are written as they are
+    assert np.load(tmp_path / "a" / "thresh.npy").tolist() == [0.5, 0.25, 0.75, 0.125, float(np.finfo(np.float32).max)]
+    idx = np.load(tmp_path / "a" / "pixel_index.npy").astype(np.int64)
+    assert len(idx) == 100 and len(np.unique(idx)) == 100 and idx.max() < n * h * w
+    for name, t in (("label", label), ("final", final), ("conf", conf), ("unc", unc)):
+        assert np.array_equal(np.load(tmp_path / "a" / (name + ".npy")), t.reshape(-1).numpy()[idx].astype(np.float32)), name
+    assert np.array_equal(np.load(tmp_path / "a" / "final_hist.npy"), job.final_hist.numpy().astype(np.float64))
+    assert np.load(tmp_path / "a" / "near_tie_pixels.npy").tolist() == [7.0]
+    assert bench.DUMP_SAMPLE_PIXELS < 2000 * 256 * 480
+    assert 4 * 4 * bench.DUMP_SAMPLE_PIXELS + 8 * bench.DUMP_SAMPLE_PIXELS <= 64 << 20     # 4 float32 maps + float64 index
+
+
+def test_reference_arm_prints_one_contract_line(tmp_path):
     env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "1", "--steps", "1",
-                        "--warmup", "1", "--ref-images", "2", "--height", "32", "--width", "48"],
+                        "--warmup", "1", "--ref-images", "2", "--height", "32", "--width", "48", "--dump-outputs", str(tmp_path)],
                        capture_output=True, text=True, env=env, timeout=600)
+    # --dump-outputs: the class weights of the last timed step, as the oracle port computes them on the same seeded inputs
+    mains, auxs = bench.make_logits_host(torch, 2, 32, 48, seed=3, pin=False)
+    _, class_array = O.multi_source_labels(mains, auxs, [O.LUTS[s] for s, _ in bench.SOURCES], "all")
+    assert os.listdir(tmp_path) == ["class_weights.npy"], p.stderr[-2000:]
+    got = np.load(tmp_path / "class_weights.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, O.class_weights_from_histogram(class_array, 'normal').numpy())
     assert p.returncode == 0, p.stderr[-2000:]
     lines = [ln for ln in p.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1, p.stdout
