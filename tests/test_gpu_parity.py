@@ -587,7 +587,7 @@ LOWRES_GEOMETRIES = [
     (2, 5, 24, 32, (24, 32), (12, 16)),             # main head already at full resolution
     (1, 8, 20, 44, (7, 11), (3, 5)),                # K = 8, large scale factors
     (2, 2, 9, 1, (5, 1), (3, 1)),                   # single column
-    (1, 5, 512, 1024, (256, 512), (128, 256)),      # stress size: only 4-row tiles fit -> an aux row gets shares from 3 tiles
+    (1, 5, 512, 1024, (256, 512), (128, 256)),      # stress size: only 2-row tiles fit -> an aux row gets shares from 3+ tiles
 ]
 
 
