@@ -81,12 +81,13 @@ def argmax_to_greenhouse(output, lut):
 
 
 def vote_threshold(num_data, thresh=None):
-    """uest_seg_multi_os.py:697-705: None/'half'/invalid -> S//2+1, 'all' -> S, int<=S -> itself."""
+    """uest_seg_multi_os.py:697-705: None/'half'/invalid -> S//2+1, 'all' -> S, int<=S -> itself.  The reference tests
+    isinstance(thresh, int), which a bool passes: True counts as 1, False as 0 (no pixel becomes the ignore class)."""
     if thresh is None or thresh == 'half':
         return num_data // 2 + 1
     if thresh == 'all':
         return num_data
-    if isinstance(thresh, int) and not isinstance(thresh, bool) and thresh <= num_data:
+    if isinstance(thresh, int) and thresh <= num_data:
         return thresh
     return num_data // 2 + 1
 

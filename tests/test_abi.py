@@ -142,3 +142,8 @@ def test_vote_threshold_follows_merge_outputs_rule():
     assert vote_threshold(3, 1) == 1 and vote_threshold(3, 3) == 3 and vote_threshold(3, 4) == 2
     assert vote_threshold(3, True) == 1 and vote_threshold(3, False) == 0
     assert vote_threshold(3, '2') == 2 and vote_threshold(4, 'nonsense') == 3 and vote_threshold(1, None) == 1
+    # the oracle's restatement follows the same rule, bool included
+    from oracle import mspl_oracle as O
+    for S in (1, 2, 3, 4, 8, 15):
+        for t in [None, 'half', 'all', '3', 'nonsense', True, False] + list(range(-1, S + 3)):
+            assert O.vote_threshold(S, t) == vote_threshold(S, t), (S, t)

@@ -28,7 +28,7 @@ def test_luts(ref):
         assert np.array_equal(getattr(ref.greenhouse, "id_%s_to_greenhouse" % name), O.LUTS[name])
 
 
-@pytest.mark.parametrize("policy", [None, "half", "all", 1, 2, 3, "3", 7])
+@pytest.mark.parametrize("policy", [None, "half", "all", 1, 2, 3, "3", 7, True, False])
 def test_label_generation_matches_reference(ref, policy):
     gen = torch.Generator().manual_seed(11)
     n, h, w = 2, 20, 36
