@@ -107,6 +107,10 @@ MSPL_API int mspl_class_order(const uint8_t* lut, int num_classes, int num_targe
  * the number of class chunks the kernel's inner loop runs for this source.  Returns the number of target groups (>= 1), or a
  * negative status. */
 MSPL_API int mspl_class_order_votes(const uint8_t* lut, int num_classes, int num_target_classes, uint32_t* vote, uint32_t* nchunk);
+/* Host-only companion: which compiled chunk shape K1 runs for this table -- 1 + the index of the listed shape (the greenhouse
+ * tables' class orders, which the kernel runs as straight-line code) whose class count, chunk count and group boundaries the
+ * table's order has, or 0 for the generic chunk loop.  Negative status on bad arguments. */
+MSPL_API int mspl_class_order_shape(const uint8_t* lut, int num_classes, int num_target_classes);
 
 /* ---- K1-lowres: K1 with the network's final upsample fused in (next-row component, SURVEY.md 8f-1) ------------------
  * Same outputs and semantics as mspl_fuse_sources, but source s hands over its logits BEFORE the final

@@ -24,6 +24,7 @@ SIGNATURES = {
                                          c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "mspl_class_order": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_vp]),
     "mspl_class_order_votes": (c_int, [c_vp, c_int, c_int, c_vp, c_vp]),
+    "mspl_class_order_shape": (c_int, [c_vp, c_int, c_int]),
     "mspl_vote_labels": (c_int, [c_vp, c_int, c_i64, c_int, c_int, c_int, c_vp, c_vp]),
     "mspl_radix_state_bytes": (c_sz, [c_int]),
     "mspl_conf_hist": (c_int, [c_vp, c_vp, c_i64, c_i64, c_int, c_vp, c_int, c_vp]),

@@ -12,6 +12,9 @@
 //                                consumer warps compute from shared memory; bytes in flight no longer cost registers
 // Both visit a source's classes grouped by target class (ClassOrder), see pixel_math.cuh.
 #pragma once
+#include <type_traits>
+#include <utility>
+
 #include "pixel_math.cuh"
 #include "bilinear.cuh"
 
@@ -540,10 +543,34 @@ struct TileWalker {
     }
 };
 
+// the value of a run-time argument or of a std::integral_constant (whose conversion operator is host-only)
+template <typename T> MSPL_DEVINL T cval(T v) { return v; }
+template <typename T, T V> MSPL_DEVINL T cval(std::integral_constant<T, V>) { return V; }
+
+// Body of listed shape SH (kSourceShapes): consume(ncls, seg, first) once per chunk, with the chunk's real class count, its
+// group-end bits and whether it is the source's first chunk as compile-time constants.
+template <int CH, int SH, typename Consume, int... I>
+MSPL_DEVINL void consume_listed_shape(Consume& consume, std::integer_sequence<int, I...>) {
+    constexpr SourceShape sh = kSourceShapes[SH];
+    (consume(std::integral_constant<int, (sh.C - I * CH < CH ? sh.C - I * CH : CH)>{}, std::integral_constant<uint32_t, sh.seg[I]>{},
+             std::bool_constant<I == 0>{}),
+     ...);
+}
+// Runs the body of listed shape `shape` (ClassOrder::shape, 1-based); false when shape is 0 or not among SH + 1.
+template <int CH, typename Consume, int... SH>
+MSPL_DEVINL bool consume_listed_shapes(uint32_t shape, Consume& consume, std::integer_sequence<int, SH...>) {
+    return ((shape == SH + 1 &&
+             (consume_listed_shape<CH, SH>(consume, std::make_integer_sequence<int, kSourceShapes[SH].nchunk>{}), true)) ||
+            ...);
+}
+
 // Producer warp of the TMA-staged kernels: walks this CTA's tiles in (tile, source, chunk) order and fills the ring.
 // s_row: per-source class visiting order ([S][256] bytes in shared memory), or nullptr for the original class order.
+// shaped: the consumers run the compiled bodies of listed shapes (ClassOrder::shape != 0), which never read the rows a tail
+// chunk lacks, so those sources' tail chunks are not padded.
 template <int NCW, int P, int CH, int NSTAGE>
-MSPL_DEVINL void tma_produce_tiles(const FuseParams& prm, float* ring, uint64_t* full, uint64_t* empty, int lane, const uint8_t* s_row) {
+MSPL_DEVINL void tma_produce_tiles(const FuseParams& prm, float* ring, uint64_t* full, uint64_t* empty, int lane, const uint8_t* s_row,
+                                   bool shaped) {
     using Cfg = TmaCfg<NCW, P, CH, NSTAGE>;
     constexpr int TP = Cfg::kTilePix;
     const int S = prm.S;
@@ -562,11 +589,12 @@ MSPL_DEVINL void tma_produce_tiles(const FuseParams& prm, float* ring, uint64_t*
             const int C = prm.C[s];
             const float* pm = prm.main[s] + (n * C) * hw + off;
             const float* pa = prm.aux[s] + (n * C) * hw + off;
+            const bool pad_tail = !(shaped && prm.order[s].shape != 0);
             for (int c0 = 0; c0 < C; c0 += CH) {
                 const int cn = min(CH, C - c0);
                 tma::mbar_wait(&empty[stage], phase ^ 1);          // all consumers released this slot
                 float* dst = ring + (size_t)stage * Cfg::kStageFloats;
-                if (cn < CH) {
+                if (cn < CH && pad_tail) {
                     // tail chunk: the class rows this source does not have are filled with kPadLogit HERE, so that the
                     // consumers' loads and math carry no predicates and exist only once in the instruction stream
                     const float4 pad = make_float4(kPadLogit, kPadLogit, kPadLogit, kPadLogit);
@@ -617,7 +645,7 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_sources_tma_kernel(con
     Tally<KT> tally;
 
     if (warp == NCW) {
-        tma_produce_tiles<NCW, P, CH, NSTAGE>(prm, ring, full, empty, lane, ts.row);
+        tma_produce_tiles<NCW, P, CH, NSTAGE>(prm, ring, full, empty, lane, ts.row, CH == kShapeChunk);
     } else {
         // ------------------------------- consumer warps -------------------------------
         const float fS = 1.0f / (float)S;
@@ -636,31 +664,41 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_sources_tma_kernel(con
             fus.reset();
             for (int s = 0; s < S; ++s) {
                 const int nchunk = (int)prm.order[s].nchunk;
-                __builtin_assume(nchunk > 0);             // every source has a class: no zero-trip guard around the chunk loop
                 SourceStats<P> st;
                 st.reset(group);
-                // one chunk: wait for its stage, copy the thread's values to registers, hand the stage back, fold
-                auto consume = [&](int chunk, bool first) {
+                // one chunk of ncls real classes: wait for its stage, copy the thread's values to registers, hand the stage
+                // back, fold.  ncls is a compile-time count; seg and first are compile-time in the listed shapes' bodies.
+                auto consume = [&](auto ncls, auto seg, auto first) {
+                    constexpr int N = decltype(ncls)::value;
                     Px<P> m[CH], a[CH];
                     tma::mbar_wait(&full[stage], phase);
                     const float* src = ring + (size_t)stage * Cfg::kStageFloats + px;
 #pragma unroll
-                    for (int j = 0; j < CH; ++j) m[j] = tma::lds_px<P>(src + j * TP);
+                    for (int j = 0; j < N; ++j) m[j] = tma::lds_px<P>(src + j * TP);
 #pragma unroll
-                    for (int j = 0; j < CH; ++j) a[j] = tma::lds_px<P>(src + (CH + j) * TP);
+                    for (int j = 0; j < N; ++j) a[j] = tma::lds_px<P>(src + (CH + j) * TP);
                     __syncwarp();
                     if (lane == 0) tma::mbar_arrive(&empty[stage]);    // values are in registers: hand the slot back
                     if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
-                    fold_chunk<P, CH>(st, m, a, first, prm.order[s].seg[chunk], Cfg::kThreads);
+                    fold_chunk<P, CH, N>(st, m, a, cval(first), cval(seg), Cfg::kThreads);
                 };
+                bool listed = false;
+                if constexpr (CH == kShapeChunk)        // warp-uniform: one straight-line body per listed shape
+                    listed = consume_listed_shapes<CH>(prm.order[s].shape, consume, std::make_integer_sequence<int, kNumSourceShapes>{});
+                if (!listed) {
+                    using AllCH = std::integral_constant<int, CH>;
+                    __builtin_assume(nchunk > 0);         // every source has a class: no zero-trip guard around the chunk loop
 #if MSPL_PEEL_FIRST == 2
-                consume(0, true);           // straight-line copy of the body without the rescale of the (empty) accumulators
+                    // straight-line copy of the body without the rescale of the (empty) accumulators
+                    consume(AllCH{}, prm.order[s].seg[0], true);
 #pragma unroll kChunkUnroll
-                for (int chunk = 1; chunk < nchunk; ++chunk) consume(chunk, false);
+                    for (int chunk = 1; chunk < nchunk; ++chunk) consume(AllCH{}, prm.order[s].seg[chunk], false);
 #else
 #pragma unroll kChunkUnroll
-                for (int chunk = 0; chunk < nchunk; ++chunk) consume(chunk, MSPL_PEEL_FIRST ? chunk == 0 : false);
+                    for (int chunk = 0; chunk < nchunk; ++chunk)
+                        consume(AllCH{}, prm.order[s].seg[chunk], MSPL_PEEL_FIRST ? chunk == 0 : false);
 #endif
+                }
                 float d[P];
                 fus.add_source(st, group, Cfg::kThreads, prm.order[s], d,
                                GlobalSlowPath<P>{prm, s, n, active ? off : 0, ts.lut + s * MSPL_MAX_SRC_CLASSES});
@@ -713,7 +751,7 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_labels_tma_kernel(cons
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     Tally<KT> tally;
     if (warp == NCW) {
-        tma_produce_tiles<NCW, P, CH, NSTAGE>(prm, ring, full, empty, lane, nullptr);
+        tma_produce_tiles<NCW, P, CH, NSTAGE>(prm, ring, full, empty, lane, nullptr, false);
     } else {
         int stage = 0;
         uint32_t phase = 0;

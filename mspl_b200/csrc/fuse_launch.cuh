@@ -21,6 +21,16 @@ inline DeviceInfo device_info() {
     return d;
 }
 
+// 1 + the index of the listed shape (kSourceShapes) that an order built for chunks of `chunk` classes has, or 0.
+inline uint32_t listed_shape(const ClassOrder& o, int C, int chunk) {
+    if (chunk != kShapeChunk) return 0;
+    for (int i = 0; i < kNumSourceShapes; ++i) {
+        const SourceShape& sh = kSourceShapes[i];
+        if (sh.C == C && sh.nchunk == (int)o.nchunk && memcmp(sh.seg, o.seg, (size_t)sh.nchunk) == 0) return (uint32_t)i + 1;
+    }
+    return 0;
+}
+
 // Class visiting order of every source for chunks of `chunk` classes (see ClassOrder in pixel_math.cuh): classes sorted by
 // (target class, class index); per chunk a byte with bit j = slot j ends its target group (chunk <= 8).
 // Needs prm.S, prm.C and prm.lut; returns false when a source has more chunks than ClassOrder::seg holds.
@@ -47,6 +57,7 @@ inline bool build_class_order(FuseParams& prm, int chunk) {
             const bool last = (i == C - 1) || prm.lut[s][o.row[i + 1]] != k;
             if (last) o.seg[i / chunk] |= (uint8_t)(1u << (i % chunk));
         }
+        o.shape = listed_shape(o, C, chunk);
     }
     return true;
 }

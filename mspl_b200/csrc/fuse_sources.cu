@@ -86,11 +86,10 @@ extern "C" const char* mspl_fuse_variant(void) {
 }
 
 // Host-only: the class visiting order K1 derives from a label table (no device work; lets the host logic be tested on CPU).
-extern "C" int mspl_class_order(const uint8_t* lut, int num_classes, int num_target_classes, uint8_t* row, uint8_t* seg,
-                                uint32_t* present) {
-    if (!lut || !row || !seg || !present || num_classes < 1 || num_classes > MSPL_MAX_SRC_CLASSES) return MSPL_ERR_BAD_ARG;
+// The class order K1 builds for one source with label table `lut`, into prm.order[0]; MSPL_OK or a negative status.
+static int class_order_of_table(const uint8_t* lut, int num_classes, int num_target_classes, FuseParams& prm) {
+    if (!lut || num_classes < 1 || num_classes > MSPL_MAX_SRC_CLASSES) return MSPL_ERR_BAD_ARG;
     if (num_target_classes < 2 || num_target_classes > MSPL_MAX_CLASSES) return MSPL_ERR_BAD_ARG;
-    FuseParams prm;
     memset(&prm, 0, sizeof(prm));
     prm.S = 1;
     prm.C[0] = num_classes;
@@ -98,7 +97,15 @@ extern "C" int mspl_class_order(const uint8_t* lut, int num_classes, int num_tar
         if (lut[c] >= num_target_classes) return MSPL_ERR_BAD_ARG;
         prm.lut[0][c] = lut[c];
     }
-    if (!build_class_order(prm, MSPL_FUSE_CH)) return MSPL_ERR_UNSUPPORTED;
+    return build_class_order(prm, MSPL_FUSE_CH) ? MSPL_OK : MSPL_ERR_UNSUPPORTED;
+}
+
+extern "C" int mspl_class_order(const uint8_t* lut, int num_classes, int num_target_classes, uint8_t* row, uint8_t* seg,
+                                uint32_t* present) {
+    if (!row || !seg || !present) return MSPL_ERR_BAD_ARG;
+    FuseParams prm;
+    const int rc = class_order_of_table(lut, num_classes, num_target_classes, prm);
+    if (rc != MSPL_OK) return rc;
     memcpy(row, prm.order[0].row, (size_t)num_classes);
     memcpy(seg, prm.order[0].seg, (size_t)((num_classes + MSPL_FUSE_CH - 1) / MSPL_FUSE_CH));
     *present = prm.order[0].present;
@@ -106,20 +113,19 @@ extern "C" int mspl_class_order(const uint8_t* lut, int num_classes, int num_tar
 }
 
 extern "C" int mspl_class_order_votes(const uint8_t* lut, int num_classes, int num_target_classes, uint32_t* vote, uint32_t* nchunk) {
-    if (!lut || !vote || !nchunk || num_classes < 1 || num_classes > MSPL_MAX_SRC_CLASSES) return MSPL_ERR_BAD_ARG;
-    if (num_target_classes < 2 || num_target_classes > MSPL_MAX_CLASSES) return MSPL_ERR_BAD_ARG;
+    if (!vote || !nchunk) return MSPL_ERR_BAD_ARG;
     FuseParams prm;
-    memset(&prm, 0, sizeof(prm));
-    prm.S = 1;
-    prm.C[0] = num_classes;
-    for (int c = 0; c < num_classes; ++c) {
-        if (lut[c] >= num_target_classes) return MSPL_ERR_BAD_ARG;
-        prm.lut[0][c] = lut[c];
-    }
-    if (!build_class_order(prm, MSPL_FUSE_CH)) return MSPL_ERR_UNSUPPORTED;
+    const int rc = class_order_of_table(lut, num_classes, num_target_classes, prm);
+    if (rc != MSPL_OK) return rc;
     memcpy(vote, prm.order[0].vote, sizeof(prm.order[0].vote));
     *nchunk = prm.order[0].nchunk;
     return (int)prm.order[0].ngroup;
+}
+
+extern "C" int mspl_class_order_shape(const uint8_t* lut, int num_classes, int num_target_classes) {
+    FuseParams prm;
+    const int rc = class_order_of_table(lut, num_classes, num_target_classes, prm);
+    return rc != MSPL_OK ? rc : (int)prm.order[0].shape;
 }
 
 extern "C" int mspl_fuse_sources(int num_sources, const float* const* main_logits, const float* const* aux_logits,

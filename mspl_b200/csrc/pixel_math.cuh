@@ -148,8 +148,10 @@ MSPL_DEVINL Px<P> pmax3(Px<P> a, Px<P> b, Px<P> c) {
     for (int p = 0; p < P; ++p) x[p] = max3(x[p], y[p], z[p]);
     return Px<P>::make(x);
 }
-template <int P, int N>
-MSPL_DEVINL Px<P> pmax_of(const Px<P> (&v)[N], Px<P> init) {
+// max of init and the first N entries of v
+template <int P, int N, int L>
+MSPL_DEVINL Px<P> pmax_of(const Px<P> (&v)[L], Px<P> init) {
+    static_assert(N <= L, "pmax_of reads past the array");
     Px<P> r = init;
     int j = 0;
 #pragma unroll
@@ -173,7 +175,27 @@ struct ClassOrder {
     uint32_t ngroup;          // number of target groups = popcount(present) (>= 1)
     uint32_t vote[MSPL_MAX_CLASSES];   // vote[i] = 1 << 4*(target class of the i-th committed group): what a source adds to a
                                        // pixel's packed vote counters (4 bits per target) when group i holds its largest z
+    uint32_t shape;           // 1 + index into kSourceShapes when (C, nchunk, seg) is a listed shape, else 0
 };
+
+// ---- compiled chunk shapes ---------------------------------------------------------------------------------------------
+// Everything the chunk loop does per source follows from (C, nchunk, seg[0..nchunk)) alone.  The shapes of the greenhouse
+// tables (data_loader/segmentation/greenhouse.py SOURCE_TABLES, at kShapeChunk classes per chunk) are listed here, and the
+// TMA kernel runs a fully unrolled body for each of them: group commits only where a group ends, no rescale on the first chunk,
+// and a tail chunk that loads and folds only its real classes (so the producer writes no padding for it).  Any other shape
+// runs the generic loop.  build_class_order sets ClassOrder::shape.
+constexpr int kShapeChunk = 5;
+constexpr int kMaxShapeChunks = 4;
+struct SourceShape {
+    int C, nchunk;
+    uint8_t seg[kMaxShapeChunks];
+};
+constexpr SourceShape kSourceShapes[] = {
+    {13, 3, {0x01, 0x0a, 0x04}},          // camvid: groups of 1, 6, 2, 4 classes
+    {20, 4, {0x01, 0x00, 0x04, 0x11}},    // cityscapes: 1, 12, 3, 4
+    {5, 1, {0x1a}},                       // forest: 2, 2, 1
+};
+constexpr int kNumSourceShapes = (int)(sizeof(kSourceShapes) / sizeof(kSourceShapes[0]));
 
 // Running per-pixel statistics of one source.
 //   Mm, Sm = sum e^{m-Mm}     Ma, Sa = sum e^{a-Ma}     T = sum e^{m-Mm} ((m-Mm) - (a-Ma))
@@ -200,16 +222,20 @@ struct SourceStats {
 // max, its exponentials are exactly 0 and (m - Mm) - (a - Ma) stays finite (0) -- the math below needs no predicates.
 constexpr float kPadLogit = -1.0e30f;
 
-// Fold the CH classes of one chunk into the running stats.  m/a hold the chunk's logits in visiting order; entries past the
-// source's last class are kPadLogit.  `first` (warp-uniform): nothing accumulated yet, skip the rescale.  seg: the chunk's
-// ClassOrder word (bit j: slot j ends its target group).  Finished groups go to st.slot, gstride entries apart.
-template <int P, int CH>
+// Fold the first N (default CH) classes of one chunk into the running stats.  m/a hold the chunk's logits in visiting order;
+// with N = CH, entries past the source's last class are kPadLogit; entries from N on are not read.  The rescale of a first
+// chunk adds exact zeros, and so do padded classes once any logit of the source lies above kPadLogit: N = the real class
+// count and N = CH with padding give the same bits, and so does either `first` on a first chunk.
+// `first` (warp-uniform): nothing accumulated yet, skip the rescale.  seg: the chunk's ClassOrder word (bit j: slot j ends
+// its target group).  Finished groups go to st.slot, gstride entries apart.
+template <int P, int CH, int N = CH>
 MSPL_DEVINL void fold_chunk(SourceStats<P>& st, const Px<P> (&m)[CH], const Px<P> (&a)[CH], bool first, uint32_t seg, int gstride) {
+    static_assert(0 < N && N <= CH, "a chunk folds 1..CH classes");
     const Px<P> half = Px<P>::splat(0.5f);
     // sweep 1: z exactly as the reference forms it (0.5*a is exact in fp32, so the fused multiply-add rounds once, just
     // like `pred + 0.5 * pred_aux`), folded into the running maximum of the current target group
 #pragma unroll
-    for (int j = 0; j < CH; ++j) {
+    for (int j = 0; j < N; ++j) {
         st.run = pmax<P>(st.run, fma(a[j], half, m[j]));
         if ((seg >> j) & 1u) {              // warp-uniform: last class of its group
             *st.slot = st.run;
@@ -217,7 +243,7 @@ MSPL_DEVINL void fold_chunk(SourceStats<P>& st, const Px<P> (&m)[CH], const Px<P
             st.run = Px<P>::splat(-INFINITY);
         }
     }
-    const Px<P> nMm = pmax_of<P, CH>(m, st.Mm), nMa = pmax_of<P, CH>(a, st.Ma);
+    const Px<P> nMm = pmax_of<P, N>(m, st.Mm), nMa = pmax_of<P, N>(a, st.Ma);
     Px<P> sm_old = Px<P>::splat(0.f), rm = sm_old, sm, sa = sm_old, sz = sm_old, t = sm_old;
     const Px<P> l2e = Px<P>::splat(kLog2e), hl2e = Px<P>::splat(0.5f * kLog2e);
     if (!first) {   // rescale what earlier chunks accumulated to the new maxima
@@ -233,7 +259,7 @@ MSPL_DEVINL void fold_chunk(SourceStats<P>& st, const Px<P> (&m)[CH], const Px<P
     // class's term: ptxas fuses a packed multiply into a following packed add whenever it sees the pair, so spelling it out
     // keeps every variant of the kernels (packed / scalar, with / without the first-chunk branch) on the same bits.
 #pragma unroll
-    for (int j = 0; j < CH; ++j) {
+    for (int j = 0; j < N; ++j) {
         const Px<P> tm = m[j] - nMm, ta = a[j] - nMa;
         const Px<P> em = pex2<P>(tm * l2e), h = pex2<P>(ta * hl2e);
         sm = (j == 0) ? fma(sm_old, rm, em) : sm + em;
