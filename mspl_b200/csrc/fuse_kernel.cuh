@@ -59,6 +59,21 @@ inline size_t fuse_tally_smem_bytes(int K, int KT, int nthreads, int P) {
     return b + sizeof(float) * (size_t)KT * nthreads * P;
 }
 
+// merge_outputs (uest_seg_multi_os.py:695-718) on one pixel's packed vote counters (4 bits per target class; classes from
+// the call's K up to KT carry no votes): the class with the most votes, the lowest one on ties (:713), and `ignore` when it
+// has fewer than vote_t votes (:716).
+template <int KT>
+MSPL_DEVINL int merge_votes(uint32_t votes, int vote_t, int ignore) {
+    int bk = 0;
+    uint32_t bc = votes & 15u;
+#pragma unroll
+    for (int k = 1; k < KT; ++k) {
+        const uint32_t c = (votes >> (4 * k)) & 15u;
+        if (c > bc) { bc = c; bk = k; }
+    }
+    return ((int)bc < vote_t) ? ignore : bk;
+}
+
 // ---- per-pixel accumulation across sources --------------------------------------------------------------------------
 // GK: per-target-class probabilities needed (policy 'prob', or a vote threshold below S); otherwise every source voted
 // for the winning label and G_s[label] is simply that source's max probability.
@@ -215,21 +230,14 @@ struct PixelFusion {
                 conf[p] = best;
                 marg[p] |= (best - second) < kNearTieMargin;
             } else {
-                int bk = 0;
-                uint32_t bc = votes[p] & 15u;
                 if (!GK && prm.vote_t == prm.S) {
                     // unanimity required ('all'): the label survives only if every source proposed it, so looking at the
                     // last proposal's count is enough -- no scan over the classes
-                    bk = (31 - __clz((int)last_vote[p])) >> 2;
-                    bc = (votes[p] >> (4 * bk)) & 15u;
+                    const int bk = (31 - __clz((int)last_vote[p])) >> 2;
+                    label[p] = ((int)((votes[p] >> (4 * bk)) & 15u) < prm.vote_t) ? ignore : bk;
                 } else {
-#pragma unroll
-                    for (int k = 1; k < K; ++k) {        // merge_outputs: most votes, lowest class on ties (:713)
-                        const uint32_t c = (votes[p] >> (4 * k)) & 15u;
-                        if (c > bc) { bc = c; bk = k; }
-                    }
+                    label[p] = merge_votes<K>(votes[p], prm.vote_t, ignore);
                 }
-                label[p] = ((int)bc < prm.vote_t) ? ignore : bk;     // (:716)
                 // every source voted for `label`, so G_s[label] is that source's max probability -- except for target class 0,
                 // which transfer_output_to_greenhouse never fills (G[0] = 0, uest_seg_multi_os.py:1340)
                 float f = (label[p] == 0) ? 0.f : cs[p];
@@ -299,6 +307,23 @@ struct Tally {
                 if (s_hist[i]) atomicAdd(prm.conf_hist + i, (unsigned long long)s_hist[i]);
     }
 };
+
+// End of a tile for the thread's P pixels off, off + 1, ... of image n (hw pixels per image): the fused label, conf and unc to
+// global memory (active: the pixels exist), then into the tallies.  inv_s = 1/S.
+template <int P, int KT, bool GK>
+MSPL_DEVINL void finish_tile(const FuseParams& prm, PixelFusion<P, KT, GK>& fus, float inv_s, Tally<KT>& tally, uint32_t* s_hist,
+                             int64_t n, int64_t hw, int64_t off, bool active) {
+    int label[P];
+    float conf[P], unc[P];
+    fus.finish(prm, inv_s, label, conf, unc);
+    if (active) {
+        const int64_t o = n * hw + off;
+        store_labels<P>(prm.label + o, label);
+        if (prm.conf) PixVec<P>::store(prm.conf + o, conf);
+        if (prm.unc) PixVec<P>::store(prm.unc + o, unc);
+    }
+    tally.template add<P>(prm, s_hist, label, conf, fus.marg, off, active);
+}
 
 // Carves the bookkeeping region (layout: fuse_tally_smem_bytes) and initialises it; the caller syncs.
 struct TallySmem {
@@ -401,16 +426,7 @@ __global__ void __launch_bounds__(THREADS, MINB) fuse_sources_direct_kernel(cons
             fus.add_source(st, group, THREADS, prm.order[s], d, GlobalSlowPath<P>{prm, s, n, off, ts.lut + s * MSPL_MAX_SRC_CLASSES});
             if (prm.kld[s] != nullptr && active) PixVec<P>::store(prm.kld[s] + n * hw + off, d);
         }
-        int label[P];
-        float conf[P], unc[P];
-        fus.finish(prm, fS, label, conf, unc);
-        if (active) {
-            const int64_t o = n * hw + off;
-            store_labels<P>(prm.label + o, label);
-            if (prm.conf) PixVec<P>::store(prm.conf + o, conf);
-            if (prm.unc) PixVec<P>::store(prm.unc + o, unc);
-        }
-        tally.template add<P>(prm, ts.hist, label, conf, fus.marg, off, active);
+        finish_tile(prm, fus, fS, tally, ts.hist, n, hw, off, active);
     }
     tally.flush(prm, ts.hist, ts.cls, THREADS);
 }
@@ -441,9 +457,7 @@ MSPL_DEVINL void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
 // hint asks for a long suspension (the producer is HBM-bound: a stage takes ~1 us to fill), so that waiting warps do not burn
 // issue slots -- and board power, which is what caps this kernel's sustained rate -- on a spin loop (6 % of all executed
 // instructions without the hint, ncu source page of round 2).
-#ifndef MSPL_MBAR_SUSPEND_NS
-#define MSPL_MBAR_SUSPEND_NS 2000
-#endif
+constexpr uint32_t kMbarSuspendNs = 2000;
 MSPL_DEVINL void mbar_wait(uint64_t* bar, uint32_t parity) {
     asm volatile(
         "{\n"
@@ -453,7 +467,7 @@ MSPL_DEVINL void mbar_wait(uint64_t* bar, uint32_t parity) {
         "@p bra DONE_%=;\n"
         "bra WAIT_%=;\n"
         "DONE_%=:\n"
-        "}\n" ::"r"(smem_addr(bar)), "r"(parity), "r"((uint32_t)MSPL_MBAR_SUSPEND_NS)
+        "}\n" ::"r"(smem_addr(bar)), "r"(parity), "r"(kMbarSuspendNs)
         : "memory");
 }
 // 1-D bulk copy global -> shared, completion counted in bytes on `bar`; streaming data: L2 evict-first hint
@@ -488,36 +502,6 @@ template <int P> MSPL_DEVINL Px<P> lds_px(const float* p) {
 
 }  // namespace tma
 
-// 0: the rescale runs on the first chunk's empty accumulators too (it evaluates to exact zeros, see SourceStats::reset) and the
-// chunk body is branch-free; 1: the first chunk of a source skips it through a branch inside the loop, whose merge costs ~20
-// register moves per chunk in the generated code; 2: the first chunk is peeled OUT of the loop as a second, straight-line copy of
-// the body without the rescale (4 MUFU and 11 packed operations less for 3 of the benchmark's 8 chunks per pixel pair).  Same bits
-// in all three.
-#ifndef MSPL_PEEL_FIRST
-#define MSPL_PEEL_FIRST 0
-#endif
-// The same choice for the fused-upsample kernel, which is bound by instruction issue, not by HBM or board power: there the
-// peeled first chunk is worth 4.5 % (1.895 -> 1.810 ms per 200 images, same-box A/B, identical outputs).
-#ifndef MSPL_LOWRES_PEEL_FIRST
-#define MSPL_LOWRES_PEEL_FIRST 2
-#endif
-// Unroll factor of its chunk loop, separately for the kernels without / with per-target probabilities (GK): 2 removes the
-// loop-carried register moves; measured +1.7 % time without GK (it spills there) and -0.4 % with GK (1.797 -> 1.790 ms per 200
-// images) -- not worth the code size, both stay at 1.
-#ifndef MSPL_LOWRES_CHUNK_UNROLL
-#define MSPL_LOWRES_CHUNK_UNROLL 1
-#endif
-#ifndef MSPL_LOWRES_CHUNK_UNROLL_GK
-#define MSPL_LOWRES_CHUNK_UNROLL_GK 1
-#endif
-
-// Unroll factor of the consumers' chunk loop (2 lets the running statistics ping-pong between two register sets instead of
-// being moved back at the end of every chunk: 164 instead of 171 instructions per chunk, 124 registers).
-#ifndef MSPL_CHUNK_UNROLL
-#define MSPL_CHUNK_UNROLL 1
-#endif
-constexpr int kChunkUnroll = MSPL_CHUNK_UNROLL;
-
 template <int NCW, int P, int CH, int NSTAGE>
 struct TmaCfg {
     static constexpr int kThreads = (NCW + 1) * 32;
@@ -529,13 +513,90 @@ struct TmaCfg {
     }
 };
 
-// (image, tile inside the image) of the tiles blockIdx.x, blockIdx.x + gridDim.x, ... without a 64-bit division per tile.
+// The shared-memory ring of the staged kernels: NSTAGE slots of stage_floats floats, then one "full" and one "empty" mbarrier
+// per slot,  [slots][full x NSTAGE][empty x NSTAGE].  The producer warp fills the slots in turn and the NCW consumer warps
+// drain them in the same order; each thread's copy of this struct holds its own position (stage, phase) in that sequence.
+template <int NCW, int NSTAGE>
+struct StageRing {
+    float* base;
+    uint64_t* full;
+    uint64_t* empty;
+    int stage_floats;
+    int stage = 0;
+    uint32_t phase = 0;
+
+    MSPL_DEVINL StageRing(unsigned char* smem, int stage_floats_)
+        : base(reinterpret_cast<float*>(smem)), full(reinterpret_cast<uint64_t*>(smem + sizeof(float) * (size_t)stage_floats_ * NSTAGE)),
+          empty(full + NSTAGE), stage_floats(stage_floats_) {}
+    // first byte after the barriers
+    MSPL_DEVINL unsigned char* end() const { return reinterpret_cast<unsigned char*>(empty + NSTAGE); }
+    // "full" completes on the producer's arrival plus the bytes of its copies, "empty" on one arrival per consumer warp.  The
+    // caller syncs the CTA before the ring is used.
+    MSPL_DEVINL void init() const {
+        if (threadIdx.x == 0) {
+            for (int i = 0; i < NSTAGE; ++i) {
+                tma::mbar_init(&full[i], 1);
+                tma::mbar_init(&empty[i], NCW);
+            }
+            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        }
+    }
+    MSPL_DEVINL float* slot() const { return base + (size_t)stage * stage_floats; }
+    MSPL_DEVINL void advance() {
+        if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
+    }
+    // consumer: wait until the current slot is filled
+    MSPL_DEVINL const float* wait_full() const {
+        tma::mbar_wait(&full[stage], phase);
+        return slot();
+    }
+    // consumer warp: its values are in registers, hand the slot back and move on
+    MSPL_DEVINL void release(int lane) {
+        __syncwarp();
+        if (lane == 0) tma::mbar_arrive(&empty[stage]);
+        advance();
+    }
+    // producer: wait until every consumer warp has released the current slot
+    MSPL_DEVINL float* wait_empty() const {
+        tma::mbar_wait(&empty[stage], phase ^ 1);
+        return slot();
+    }
+    // producer warp: announce `bytes` of bulk copies into the current slot (a release: it publishes what the warp wrote into the
+    // slot before, the padding); the copies complete on the returned barrier.  advance() once they are issued.
+    MSPL_DEVINL uint64_t* expect(int lane, uint32_t bytes) const {
+        __syncwarp();
+        if (lane == 0) tma::mbar_arrive_expect_tx(&full[stage], bytes);
+        return &full[stage];
+    }
+};
+
+// Producer warp, tail chunk of cn < CH classes: the class rows the source does not have are filled with kPadLogit HERE, so that
+// the consumers' loads and math carry no predicates and exist only once in the instruction stream.  n4: float4 per row of a
+// head; stride: floats from one class row (block) of a head to the next; the aux head's rows start at aux_base.
+template <int CH>
+MSPL_DEVINL void pad_tail_rows(float* dst, int cn, int lane, int main_n4, int main_stride, int aux_base, int aux_n4, int aux_stride) {
+    const float4 pad = make_float4(kPadLogit, kPadLogit, kPadLogit, kPadLogit);
+    for (int j = cn; j < CH; ++j) {
+        for (int i = lane; i < main_n4; i += 32) reinterpret_cast<float4*>(dst + j * main_stride)[i] = pad;
+        for (int i = lane; i < aux_n4; i += 32) reinterpret_cast<float4*>(dst + aux_base + j * aux_stride)[i] = pad;
+    }
+    __threadfence_block();
+}
+
+// This CTA's tiles blockIdx.x, blockIdx.x + gridDim.x, ... of TP consecutive pixels of one image (the last tile of an image may
+// be shorter), as (image, tile inside the image), without a 64-bit division per tile.  The producer and the consumers of a ring
+// walk the same sequence: for (TileWalker t(hw, TP); t.image < n_img; t.next()).
 struct TileWalker {
-    int64_t image, tile_in_image;
-    int64_t step_images, step_tiles, tpi;
-    MSPL_DEVINL TileWalker(int64_t first, int64_t stride, int64_t tiles_per_image)
-        : image(first / tiles_per_image), tile_in_image(first % tiles_per_image), step_images(stride / tiles_per_image),
-          step_tiles(stride % tiles_per_image), tpi(tiles_per_image) {}
+    int64_t tpi, image, tile_in_image;
+    uint32_t step_images, step_tiles;
+    MSPL_DEVINL TileWalker(int64_t hw, int tile_pix) : tpi((hw + tile_pix - 1) / tile_pix) {
+        // blockIdx.x < gridDim.x < 2^31: a 32-bit division, with tiles per image beyond 32 bits clamped (same quotients)
+        const uint32_t t = (uint32_t)(tpi < 0xffffffffll ? tpi : 0xffffffffll);
+        image = blockIdx.x / t;
+        tile_in_image = blockIdx.x % t;
+        step_images = gridDim.x / t;
+        step_tiles = gridDim.x % t;
+    }
     MSPL_DEVINL void next() {
         image += step_images;
         tile_in_image += step_tiles;
@@ -564,26 +625,19 @@ MSPL_DEVINL bool consume_listed_shapes(uint32_t shape, Consume& consume, std::in
             ...);
 }
 
-// Producer warp of the TMA-staged kernels: walks this CTA's tiles in (tile, source, chunk) order and fills the ring.
+// Producer warp of the full-resolution TMA kernels: walks this CTA's tiles in (tile, source, chunk) order and fills the ring.
 // s_row: per-source class visiting order ([S][256] bytes in shared memory), or nullptr for the original class order.
 // shaped: the consumers run the compiled bodies of listed shapes (ClassOrder::shape != 0), which never read the rows a tail
 // chunk lacks, so those sources' tail chunks are not padded.
 template <int NCW, int P, int CH, int NSTAGE>
-MSPL_DEVINL void tma_produce_tiles(const FuseParams& prm, float* ring, uint64_t* full, uint64_t* empty, int lane, const uint8_t* s_row,
-                                   bool shaped) {
-    using Cfg = TmaCfg<NCW, P, CH, NSTAGE>;
-    constexpr int TP = Cfg::kTilePix;
+MSPL_DEVINL void tma_produce_tiles(const FuseParams& prm, StageRing<NCW, NSTAGE>& ring, int lane, const uint8_t* s_row, bool shaped) {
+    constexpr int TP = TmaCfg<NCW, P, CH, NSTAGE>::kTilePix;
     const int S = prm.S;
     const int64_t hw = prm.hw;
-    const int64_t tpi = (hw + TP - 1) / TP;
-    const int64_t n_tiles = prm.n_img * tpi;
     const uint64_t policy = tma::evict_first_policy();
-    int stage = 0;
-    uint32_t phase = 0;
-    TileWalker walk(blockIdx.x, gridDim.x, tpi);
-    for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, walk.next()) {
-        const int64_t n = walk.image;
-        const int64_t off = walk.tile_in_image * TP;
+    for (TileWalker t(hw, TP); t.image < prm.n_img; t.next()) {
+        const int64_t n = t.image;
+        const int64_t off = t.tile_in_image * TP;
         const uint32_t row_bytes = (uint32_t)((hw - off < TP ? hw - off : TP) * sizeof(float));
         for (int s = 0; s < S; ++s) {
             const int C = prm.C[s];
@@ -592,28 +646,16 @@ MSPL_DEVINL void tma_produce_tiles(const FuseParams& prm, float* ring, uint64_t*
             const bool pad_tail = !(shaped && prm.order[s].shape != 0);
             for (int c0 = 0; c0 < C; c0 += CH) {
                 const int cn = min(CH, C - c0);
-                tma::mbar_wait(&empty[stage], phase ^ 1);          // all consumers released this slot
-                float* dst = ring + (size_t)stage * Cfg::kStageFloats;
-                if (cn < CH && pad_tail) {
-                    // tail chunk: the class rows this source does not have are filled with kPadLogit HERE, so that the
-                    // consumers' loads and math carry no predicates and exist only once in the instruction stream
-                    const float4 pad = make_float4(kPadLogit, kPadLogit, kPadLogit, kPadLogit);
-                    for (int j = cn; j < CH; ++j)
-                        for (int i = lane; i < TP / 4; i += 32) {
-                            reinterpret_cast<float4*>(dst + j * TP)[i] = pad;
-                            reinterpret_cast<float4*>(dst + (CH + j) * TP)[i] = pad;
-                        }
-                    __threadfence_block();
-                }
-                __syncwarp();
-                if (lane == 0) tma::mbar_arrive_expect_tx(&full[stage], 2 * cn * row_bytes);   // release: publishes the padding too
+                float* dst = ring.wait_empty();
+                if (cn < CH && pad_tail) pad_tail_rows<CH>(dst, cn, lane, TP / 4, TP, CH * TP, TP / 4, TP);
+                uint64_t* full = ring.expect(lane, 2 * cn * row_bytes);
                 for (int j = lane; j < 2 * cn; j += 32) {
                     const int head = j >= cn, c = head ? j - cn : j;
                     const int cls = s_row ? (int)s_row[s * MSPL_MAX_SRC_CLASSES + c0 + c] : c0 + c;
                     const float* src = (head ? pa : pm) + (int64_t)cls * hw;
-                    tma::bulk_g2s(dst + (head * CH + c) * TP, src, row_bytes, &full[stage], policy);
+                    tma::bulk_g2s(dst + (head * CH + c) * TP, src, row_bytes, full, policy);
                 }
-                if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
+                ring.advance();
             }
         }
     }
@@ -624,41 +666,28 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_sources_tma_kernel(con
     using Cfg = TmaCfg<NCW, P, CH, NSTAGE>;
     constexpr int TP = Cfg::kTilePix;
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    float* ring = reinterpret_cast<float*>(smem_raw);
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + Cfg::kRingBytes);
-    uint64_t* empty = full + NSTAGE;
-    const TallySmem ts = tally_smem_init(prm, smem_raw + Cfg::kRingBytes + 2 * NSTAGE * sizeof(uint64_t), Cfg::kThreads, KT * Cfg::kThreads * P);
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < NSTAGE; ++i) {
-            tma::mbar_init(&full[i], 1);
-            tma::mbar_init(&empty[i], NCW);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    StageRing<NCW, NSTAGE> ring(smem_raw, Cfg::kStageFloats);
+    const TallySmem ts = tally_smem_init(prm, ring.end(), Cfg::kThreads, KT * Cfg::kThreads * P);
+    ring.init();
     __syncthreads();
 
     const int S = prm.S;
     const int64_t hw = prm.hw;
-    const int64_t tpi = (hw + TP - 1) / TP;            // tiles per image (the last one may be partial)
-    const int64_t n_tiles = prm.n_img * tpi;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     Tally<KT> tally;
 
     if (warp == NCW) {
-        tma_produce_tiles<NCW, P, CH, NSTAGE>(prm, ring, full, empty, lane, ts.row, CH == kShapeChunk);
+        tma_produce_tiles<NCW, P, CH, NSTAGE>(prm, ring, lane, ts.row, CH == kFuseChunk);
     } else {
         // ------------------------------- consumer warps -------------------------------
         const float fS = 1.0f / (float)S;
-        int stage = 0;
-        uint32_t phase = 0;
         const int px = (warp * 32 + lane) * P;          // this thread's first pixel inside the tile
         Px<P>* group = reinterpret_cast<Px<P>*>(ts.group) + threadIdx.x;
         bool any_kld = false;
         for (int s = 0; s < S; ++s) any_kld |= prm.kld[s] != nullptr;
-        TileWalker walk(blockIdx.x, gridDim.x, tpi);
-        for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, walk.next()) {
-            const int64_t n = walk.image;
-            const int64_t off = walk.tile_in_image * TP + px;
+        for (TileWalker t(hw, TP); t.image < prm.n_img; t.next()) {
+            const int64_t n = t.image;
+            const int64_t off = t.tile_in_image * TP + px;
             const bool active = off < hw;                 // partial last tile: the ring holds stale values past the image
             PixelFusion<P, KT, GK> fus;
             fus.reset();
@@ -671,33 +700,28 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_sources_tma_kernel(con
                 auto consume = [&](auto ncls, auto seg, auto first) {
                     constexpr int N = decltype(ncls)::value;
                     Px<P> m[CH], a[CH];
-                    tma::mbar_wait(&full[stage], phase);
-                    const float* src = ring + (size_t)stage * Cfg::kStageFloats + px;
+                    const float* src = ring.wait_full() + px;
 #pragma unroll
                     for (int j = 0; j < N; ++j) m[j] = tma::lds_px<P>(src + j * TP);
 #pragma unroll
                     for (int j = 0; j < N; ++j) a[j] = tma::lds_px<P>(src + (CH + j) * TP);
-                    __syncwarp();
-                    if (lane == 0) tma::mbar_arrive(&empty[stage]);    // values are in registers: hand the slot back
-                    if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
+                    ring.release(lane);
                     fold_chunk<P, CH, N>(st, m, a, cval(first), cval(seg), Cfg::kThreads);
                 };
                 bool listed = false;
-                if constexpr (CH == kShapeChunk)        // warp-uniform: one straight-line body per listed shape
+                if constexpr (CH == kFuseChunk)         // warp-uniform: one straight-line body per listed shape
                     listed = consume_listed_shapes<CH>(prm.order[s].shape, consume, std::make_integer_sequence<int, kNumSourceShapes>{});
                 if (!listed) {
+                    // Any other shape: the rescale runs on the first chunk's empty accumulators too (it evaluates to exact zeros,
+                    // see SourceStats::reset), so the loop body is branch-free.  Measured and not kept: skipping it through a
+                    // branch inside the loop (the merge costs ~20 register moves per chunk); peeling the first chunk out of the
+                    // loop (4 MUFU and 11 packed operations less for 3 of the benchmark's 8 chunks per pixel pair, +1 % in bursts
+                    // and nothing under the power limit); unrolling by 2 (164 instead of 171 instructions per chunk, 124
+                    // registers).  Same bits in all of them.
                     using AllCH = std::integral_constant<int, CH>;
                     __builtin_assume(nchunk > 0);         // every source has a class: no zero-trip guard around the chunk loop
-#if MSPL_PEEL_FIRST == 2
-                    // straight-line copy of the body without the rescale of the (empty) accumulators
-                    consume(AllCH{}, prm.order[s].seg[0], true);
-#pragma unroll kChunkUnroll
-                    for (int chunk = 1; chunk < nchunk; ++chunk) consume(AllCH{}, prm.order[s].seg[chunk], false);
-#else
-#pragma unroll kChunkUnroll
-                    for (int chunk = 0; chunk < nchunk; ++chunk)
-                        consume(AllCH{}, prm.order[s].seg[chunk], MSPL_PEEL_FIRST ? chunk == 0 : false);
-#endif
+#pragma unroll 1
+                    for (int chunk = 0; chunk < nchunk; ++chunk) consume(AllCH{}, prm.order[s].seg[chunk], false);
                 }
                 float d[P];
                 fus.add_source(st, group, Cfg::kThreads, prm.order[s], d,
@@ -706,16 +730,7 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_sources_tma_kernel(con
                     if (prm.kld[s] != nullptr && active) PixVec<P>::store(prm.kld[s] + n * hw + off, d);
                 }
             }
-            int label[P];
-            float conf[P], unc[P];
-            fus.finish(prm, fS, label, conf, unc);
-            if (active) {
-                const int64_t o = n * hw + off;
-                store_labels<P>(prm.label + o, label);
-                if (prm.conf) PixVec<P>::store(prm.conf + o, conf);
-                if (prm.unc) PixVec<P>::store(prm.unc + o, unc);
-            }
-            tally.template add<P>(prm, ts.hist, label, conf, fus.marg, off, active);
+            finish_tile(prm, fus, fS, tally, ts.hist, n, hw, off, active);
         }
     }
     tally.flush(prm, ts.hist, ts.cls, Cfg::kThreads);
@@ -732,33 +747,21 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_labels_tma_kernel(cons
     using Cfg = TmaCfg<NCW, P, CH, NSTAGE>;
     constexpr int TP = Cfg::kTilePix;
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    float* ring = reinterpret_cast<float*>(smem_raw);
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + Cfg::kRingBytes);
-    uint64_t* empty = full + NSTAGE;
-    const TallySmem ts = tally_smem_init(prm, smem_raw + Cfg::kRingBytes + 2 * NSTAGE * sizeof(uint64_t), Cfg::kThreads);
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < NSTAGE; ++i) {
-            tma::mbar_init(&full[i], 1);
-            tma::mbar_init(&empty[i], NCW);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    StageRing<NCW, NSTAGE> ring(smem_raw, Cfg::kStageFloats);
+    const TallySmem ts = tally_smem_init(prm, ring.end(), Cfg::kThreads);
+    ring.init();
     __syncthreads();
     const int S = prm.S;
     const int64_t hw = prm.hw;
-    const int64_t tpi = (hw + TP - 1) / TP;
-    const int64_t n_tiles = prm.n_img * tpi;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     Tally<KT> tally;
     if (warp == NCW) {
-        tma_produce_tiles<NCW, P, CH, NSTAGE>(prm, ring, full, empty, lane, nullptr, false);
+        tma_produce_tiles<NCW, P, CH, NSTAGE>(prm, ring, lane, nullptr, false);
     } else {
-        int stage = 0;
-        uint32_t phase = 0;
         const int px = (warp * 32 + lane) * P;
-        for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            const int64_t n = tile / tpi;
-            const int64_t off = (tile - n * tpi) * TP + px;
+        for (TileWalker t(hw, TP); t.image < prm.n_img; t.next()) {
+            const int64_t n = t.image;
+            const int64_t off = t.tile_in_image * TP + px;
             const bool active = off < hw;
             uint32_t votes[P];
 #pragma unroll
@@ -772,15 +775,12 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_labels_tma_kernel(cons
 #pragma unroll 1
                 for (int c0 = 0; c0 < C; c0 += CH) {
                     float m[CH][P], a[CH][P];
-                    tma::mbar_wait(&full[stage], phase);
-                    const float* src = ring + (size_t)stage * Cfg::kStageFloats + px;
+                    const float* src = ring.wait_full() + px;
 #pragma unroll
                     for (int j = 0; j < CH; ++j) tma::lds<P>(src + j * TP, m[j]);
 #pragma unroll
                     for (int j = 0; j < CH; ++j) tma::lds<P>(src + (CH + j) * TP, a[j]);
-                    __syncwarp();
-                    if (lane == 0) tma::mbar_arrive(&empty[stage]);
-                    if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
+                    ring.release(lane);
 #pragma unroll
                     for (int j = 0; j < CH; ++j)
 #pragma unroll
@@ -798,14 +798,7 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_labels_tma_kernel(cons
             bool marg[P];
 #pragma unroll
             for (int p = 0; p < P; ++p) {
-                int bk = 0;
-                uint32_t bc = votes[p] & 15u;
-#pragma unroll
-                for (int k = 1; k < KT; ++k) {        // merge_outputs: most votes, lowest class on ties (:713)
-                    const uint32_t c = (votes[p] >> (4 * k)) & 15u;
-                    if (c > bc) { bc = c; bk = k; }
-                }
-                label[p] = ((int)bc < prm.vote_t) ? prm.ignore : bk;     // (:716)
+                label[p] = merge_votes<KT>(votes[p], prm.vote_t, prm.ignore);
                 conf[p] = 0.f;
                 marg[p] = false;
             }
@@ -824,8 +817,8 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_labels_tma_kernel(cons
 //   A tile is TP consecutive output pixels (row-major) of one image.  For every class of the chunk the producer copies
 //   the block of source rows the tile's output rows interpolate from (whole rows, one bulk copy per class and head).
 //   Source coordinates and weights follow ATen's upsample_bilinear2d (src = dst * (in-1)/(out-1); i = (int)src;
-//   lambda = src - i); val = h0*(w0*v00 + w1*v01) + h1*(w0*v10 + w1*v11), evaluated for the thread's two pixels at once
-//   with packed multiplies / fmas: per class, head and PAIR of pixels 8 shared-memory loads + 6 packed instructions.
+//   lambda = src - i); val = W00*v00 + W01*v01 + W10*v10 + W11*v11 (see PackedTaps), evaluated for the thread's two pixels at
+//   once with packed multiplies / fmas: per class, head and PAIR of pixels 8 shared-memory loads + 4 packed instructions.
 //   (A separable variant -- one warp-specialised vertical pass into a second shared-memory ring, then a 2-tap horizontal
 //   pass per pixel -- was built and measured in round 2: 4.45 ms per 200 images with two blender warps against 2.08 ms
 //   for the round-1 four-tap kernel; the vertical pass's address arithmetic and its extra hand-off cost more than the
@@ -846,15 +839,16 @@ static __device__ __noinline__ float lowres_logit_global(const float* __restrict
 }
 template <int P>
 struct LowresSlowPath {
-    const float* gm;      // class 0 of this image's main / aux head
+    const float* gm;      // class 0 of image 0's main / aux head (the image's own is formed inside the rare branch)
     const float* ga;
+    int64_t n;
     int C, hm, wm, ha, wa;
     float rhm, rwm, rha, rwa;
     int yy[P], xx[P];
     const uint8_t* lut;
     MSPL_DEVINL float z(int c, int p) const {
-        return fmaf(0.5f, lowres_logit_global(ga + (int64_t)c * ha * wa, ha, wa, rha, rwa, yy[p], xx[p]),
-                    lowres_logit_global(gm + (int64_t)c * hm * wm, hm, wm, rhm, rwm, yy[p], xx[p]));
+        return fmaf(0.5f, lowres_logit_global(ga + (n * C + c) * ha * wa, ha, wa, rha, rwa, yy[p], xx[p]),
+                    lowres_logit_global(gm + (n * C + c) * hm * wm, hm, wm, rhm, rwm, yy[p], xx[p]));
     }
     MSPL_DEVINL float pmax(int p, float Mz) const {
         float s = 0.f;
@@ -881,22 +875,15 @@ struct LowresSlowPath {
 // past the row: the next row, or finite slack inside the stage, which lowres_plan provides and the kernel zero-fills once) is
 // multiplied by an exact zero.  Four registers of offsets instead of eight per head keeps the taps resident across the chunk
 // loop -- with eight the compiler re-derived them from the pixel coordinates in every chunk (~70 instructions).
-// MSPL_LOWRES_FOUR_WEIGHTS = 1 (default): the bilinear sample is evaluated as one chain over the four taps with the products of the
-// vertical and horizontal weights formed once per tile, W00*v00 + W01*v01 + W10*v10 + W11*v11 (1 packed multiply + 3 packed fmas per
-// class, head and pixel pair); 0: ATen's nesting h0*(w0*v00 + w1*v01) + h1*(w0*v10 + w1*v11) (6 packed instructions).  The two
-// differ in the last ulp of the interpolated logit, like the kernel and ATen do anyway (the parity definition of this row, DESIGN.md
-// section 4, excuses exactly that); the kernel is bound by instruction issue, so the 20 instructions per chunk are worth ~5 %.
-#ifndef MSPL_LOWRES_FOUR_WEIGHTS
-#define MSPL_LOWRES_FOUR_WEIGHTS 1
-#endif
+// The bilinear sample is evaluated as one chain over the four taps with the products of the vertical and horizontal weights
+// formed once per tile, W00*v00 + W01*v01 + W10*v10 + W11*v11 (1 packed multiply + 3 packed fmas per class, head and pixel pair),
+// not in ATen's nesting h0*(w0*v00 + w1*v01) + h1*(w0*v10 + w1*v11) (6 packed instructions).  The two differ in the last ulp of
+// the interpolated logit, like the kernel and ATen do anyway (the parity definition of this row, DESIGN.md section 4, excuses
+// exactly that); the kernel is bound by instruction issue, so the 20 instructions per chunk are worth ~5 %.
 template <int P>
 struct PackedTaps {
     int o0[P], o1[P];
-#if MSPL_LOWRES_FOUR_WEIGHTS
     Px<P> w00, w01, w10, w11;
-#else
-    Px<P> w0, w1, h0, h1;
-#endif
     MSPL_DEVINL void set(const int (&yy)[P], const int (&xx)[P], int hin, int win, float rh, float rw, int first_row) {
         float fw0[P], fw1[P], fh0[P], fh1[P];
 #pragma unroll
@@ -907,12 +894,8 @@ struct PackedTaps {
             const bool last_col = t.dx == 0;
             fw0[p] = last_col ? 1.0f : t.w0; fw1[p] = last_col ? 0.0f : t.w1; fh0[p] = t.h0; fh1[p] = t.h1;
         }
-#if MSPL_LOWRES_FOUR_WEIGHTS
         const Px<P> w0 = Px<P>::make(fw0), w1 = Px<P>::make(fw1), h0 = Px<P>::make(fh0), h1 = Px<P>::make(fh1);
         w00 = h0 * w0; w01 = h0 * w1; w10 = h1 * w0; w11 = h1 * w1;
-#else
-        w0 = Px<P>::make(fw0); w1 = Px<P>::make(fw1); h0 = Px<P>::make(fh0); h1 = Px<P>::make(fh1);
-#endif
     }
     template <int D>
     MSPL_DEVINL Px<P> gather(const float* __restrict__ s, const int (&o)[P]) const {
@@ -922,61 +905,43 @@ struct PackedTaps {
         return Px<P>::make(v);
     }
     MSPL_DEVINL Px<P> interpolate(const float* __restrict__ s) const {
-#if MSPL_LOWRES_FOUR_WEIGHTS
         Px<P> acc = w00 * gather<0>(s, o0);
         acc = fma(w01, gather<1>(s, o0), acc);
         acc = fma(w10, gather<0>(s, o1), acc);
         return fma(w11, gather<1>(s, o1), acc);
-#else
-        const Px<P> top = fma(w1, gather<1>(s, o0), w0 * gather<0>(s, o0));
-        const Px<P> bot = fma(w1, gather<1>(s, o1), w0 * gather<0>(s, o1));
-        return fma(h1, bot, h0 * top);
-#endif
     }
 };
 
 template <int NCW, int P, int CH, int NSTAGE, int KT, bool GK, int MS = 0, int AS = 0>
 __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_sources_lowres_kernel(const __grid_constant__ FuseParams prm) {
-    constexpr int kThreads = (NCW + 1) * 32;
-    constexpr int TP = NCW * 32 * P;
+    using Cfg = TmaCfg<NCW, P, CH, NSTAGE>;
+    constexpr int kThreads = Cfg::kThreads;
+    constexpr int TP = Cfg::kTilePix;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const LowresGeom& lr = prm.lr;
     const int main_stride = MS ? MS : lr.main_cls_stride, aux_stride = AS ? AS : lr.aux_cls_stride;
     const int aux_base = MS ? CH * MS : lr.aux_base;
     const int stage_floats = (MS && AS) ? CH * (MS + AS) : lr.stage_floats;
-    float* ring = reinterpret_cast<float*>(smem_raw);
-    const size_t ring_bytes = sizeof(float) * (size_t)stage_floats * NSTAGE;
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + ring_bytes);
-    uint64_t* empty = full + NSTAGE;
-    const TallySmem ts = tally_smem_init(prm, smem_raw + ring_bytes + 2 * NSTAGE * sizeof(uint64_t), kThreads, KT * kThreads * P);
+    StageRing<NCW, NSTAGE> ring(smem_raw, stage_floats);
+    const TallySmem ts = tally_smem_init(prm, ring.end(), kThreads, KT * kThreads * P);
     // the +1-float reads of PackedTaps may touch floats no copy ever wrote (slack between class blocks): make them finite once
-    for (int i = threadIdx.x; i < stage_floats * NSTAGE; i += kThreads) ring[i] = 0.f;
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < NSTAGE; ++i) {
-            tma::mbar_init(&full[i], 1);
-            tma::mbar_init(&empty[i], NCW);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    for (int i = threadIdx.x; i < stage_floats * NSTAGE; i += kThreads) ring.base[i] = 0.f;
+    ring.init();
     // generic-proxy writes above must be ordered before the async-proxy (bulk copy) writes into the same shared memory
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     __syncthreads();
 
     const int S = prm.S, H = lr.H, W = lr.W;
     const int64_t hw = prm.hw;
-    const int64_t tpi = (hw + TP - 1) / TP;
-    const int64_t n_tiles = prm.n_img * tpi;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     Tally<KT> tally;
 
     if (warp == NCW) {
         // ------------------------------- producer warp -------------------------------
         const uint64_t policy = tma::evict_first_policy();
-        int stage = 0;
-        uint32_t phase = 0;
-        for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            const int64_t n = tile / tpi;
-            const int64_t off = (tile - n * tpi) * TP;
+        for (TileWalker t(hw, TP); t.image < prm.n_img; t.next()) {
+            const int64_t n = t.image;
+            const int64_t off = t.tile_in_image * TP;
             const int y_first = (int)(off / W);
             const int64_t last = (off + TP < hw ? off + TP : hw) - 1;
             const int y_last = (int)(last / W);
@@ -991,39 +956,27 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_sources_lowres_kernel(
                 const float* pa = prm.aux[s] + ((n * C) * ha + a0) * wa;
                 for (int c0 = 0; c0 < C; c0 += CH) {
                     const int cn = min(CH, C - c0);
-                    tma::mbar_wait(&empty[stage], phase ^ 1);
-                    float* dst = ring + (size_t)stage * stage_floats;
-                    if (cn < CH) {      // pad the class blocks a tail chunk lacks (see fuse_sources_tma_kernel)
-                        const float4 pad = make_float4(kPadLogit, kPadLogit, kPadLogit, kPadLogit);
-                        for (int j = cn; j < CH; ++j) {
-                            for (int i = lane; i < (int)(mbytes / 16); i += 32) reinterpret_cast<float4*>(dst + j * main_stride)[i] = pad;
-                            for (int i = lane; i < (int)(abytes / 16); i += 32)
-                                reinterpret_cast<float4*>(dst + aux_base + j * aux_stride)[i] = pad;
-                        }
-                        __threadfence_block();
-                    }
-                    __syncwarp();
-                    if (lane == 0) tma::mbar_arrive_expect_tx(&full[stage], cn * (mbytes + abytes));
+                    float* dst = ring.wait_empty();
+                    if (cn < CH) pad_tail_rows<CH>(dst, cn, lane, (int)(mbytes / 16), main_stride, aux_base, (int)(abytes / 16), aux_stride);
+                    uint64_t* full = ring.expect(lane, cn * (mbytes + abytes));
                     for (int j = lane; j < 2 * cn; j += 32) {
                         const int head = j >= cn, c = head ? j - cn : j;
                         const int cls = ts.row[s * MSPL_MAX_SRC_CLASSES + c0 + c];
-                        if (head) tma::bulk_g2s(dst + aux_base + c * aux_stride, pa + (int64_t)cls * ha * wa, abytes, &full[stage], policy);
-                        else tma::bulk_g2s(dst + c * main_stride, pm + (int64_t)cls * hm * wm, mbytes, &full[stage], policy);
+                        if (head) tma::bulk_g2s(dst + aux_base + c * aux_stride, pa + (int64_t)cls * ha * wa, abytes, full, policy);
+                        else tma::bulk_g2s(dst + c * main_stride, pm + (int64_t)cls * hm * wm, mbytes, full, policy);
                     }
-                    if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
+                    ring.advance();
                 }
             }
         }
     } else {
         // ------------------------------- consumer warps -------------------------------
         const float inv_s = 1.0f / (float)S;
-        int stage = 0;
-        uint32_t phase = 0;
         const int px = (warp * 32 + lane) * P;
         Px<P>* group = reinterpret_cast<Px<P>*>(ts.group) + threadIdx.x;
-        for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            const int64_t n = tile / tpi;
-            const int64_t tile_off = (tile - n * tpi) * TP;
+        for (TileWalker t(hw, TP); t.image < prm.n_img; t.next()) {
+            const int64_t n = t.image;
+            const int64_t tile_off = t.tile_in_image * TP;
             const int64_t off = tile_off + px;
             const bool active = off < hw;
             const int y_first = (int)(tile_off / W);
@@ -1049,47 +1002,34 @@ __global__ void __launch_bounds__((NCW + 1) * 32, 1) fuse_sources_lowres_kernel(
                 st.reset(group);
                 const int nchunk = (int)prm.order[s].nchunk;
                 __builtin_assume(nchunk > 0);
-                constexpr int kUnroll = GK ? MSPL_LOWRES_CHUNK_UNROLL_GK : MSPL_LOWRES_CHUNK_UNROLL;
                 auto consume = [&](int chunk, bool first) {
                     Px<P> m[CH], a[CH];
-                    tma::mbar_wait(&full[stage], phase);
-                    const float* src = ring + (size_t)stage * stage_floats;
+                    const float* src = ring.wait_full();
 #pragma unroll
                     for (int j = 0; j < CH; ++j) {
                         m[j] = tm.interpolate(src + j * main_stride);
                         a[j] = ta.interpolate(src + aux_base + j * aux_stride);
                     }
-                    __syncwarp();
-                    if (lane == 0) tma::mbar_arrive(&empty[stage]);
-                    if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
+                    ring.release(lane);
                     fold_chunk<P, CH>(st, m, a, first, prm.order[s].seg[chunk], kThreads);
                 };
-#if MSPL_LOWRES_PEEL_FIRST == 2
+                // The first chunk is peeled out of the loop as a straight-line copy of the body without the rescale of the empty
+                // accumulators.  This kernel is bound by instruction issue, not by HBM or board power, so that is worth 4.5 %
+                // here (1.895 -> 1.810 ms per 200 images, same-box A/B, identical outputs).  Unrolling the loop by 2 removes its
+                // loop-carried register moves but measured +1.7 % time without GK (it spills there) and -0.4 % with GK (1.797
+                // -> 1.790 ms per 200 images): not worth the code size.
                 consume(0, true);
-#pragma unroll kUnroll
+#pragma unroll 1
                 for (int chunk = 1; chunk < nchunk; ++chunk) consume(chunk, false);
-#else
-#pragma unroll kUnroll
-                for (int chunk = 0; chunk < nchunk; ++chunk) consume(chunk, MSPL_LOWRES_PEEL_FIRST ? chunk == 0 : false);
-#endif
                 float d[P];
-                LowresSlowPath<P> slow{prm.main[s] + (n * C) * hm * wm, prm.aux[s] + (n * C) * ha * wa, C, hm, wm, ha, wa,
+                LowresSlowPath<P> slow{prm.main[s], prm.aux[s], n, C, hm, wm, ha, wa,
                                        rhm, rwm, rha, rwa, {}, {}, ts.lut + s * MSPL_MAX_SRC_CLASSES};
 #pragma unroll
                 for (int p = 0; p < P; ++p) { slow.yy[p] = yy[p]; slow.xx[p] = xx[p]; }
                 fus.add_source(st, group, kThreads, prm.order[s], d, slow);
                 if (prm.kld[s] != nullptr && active) PixVec<P>::store(prm.kld[s] + n * hw + off, d);
             }
-            int label[P];
-            float conf[P], unc[P];
-            fus.finish(prm, inv_s, label, conf, unc);
-            if (active) {
-                const int64_t o = n * hw + off;
-                store_labels<P>(prm.label + o, label);
-                if (prm.conf) PixVec<P>::store(prm.conf + o, conf);
-                if (prm.unc) PixVec<P>::store(prm.unc + o, unc);
-            }
-            tally.template add<P>(prm, ts.hist, label, conf, fus.marg, off, active);
+            finish_tile(prm, fus, inv_s, tally, ts.hist, n, hw, off, active);
         }
     }
     tally.flush(prm, ts.hist, ts.cls, kThreads);

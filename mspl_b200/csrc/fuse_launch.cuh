@@ -23,7 +23,7 @@ inline DeviceInfo device_info() {
 
 // 1 + the index of the listed shape (kSourceShapes) that an order built for chunks of `chunk` classes has, or 0.
 inline uint32_t listed_shape(const ClassOrder& o, int C, int chunk) {
-    if (chunk != kShapeChunk) return 0;
+    if (chunk != kFuseChunk) return 0;
     for (int i = 0; i < kNumSourceShapes; ++i) {
         const SourceShape& sh = kSourceShapes[i];
         if (sh.C == C && sh.nchunk == (int)o.nchunk && memcmp(sh.seg, o.seg, (size_t)sh.nchunk) == 0) return (uint32_t)i + 1;
@@ -80,10 +80,10 @@ int launch_fuse_direct(Kern kern, const FuseParams& prm, int KT, cudaStream_t st
     return launch_status();
 }
 
-// One CTA per SM (the shared-memory ring fills the SM), striding over the tiles.
+// The staged kernels (TMA, K1-lowres): one CTA per SM (the shared-memory ring fills the SM), striding over the tiles of
+// Cfg::kTilePix pixels; smem: the kernel's dynamic shared memory (TmaCfg::smem_bytes, lowres_plan).
 template <typename Cfg, typename Kern>
-int launch_fuse_tma(Kern kern, const FuseParams& prm, int KT, cudaStream_t stream) {
-    const size_t smem = Cfg::smem_bytes(prm.K, KT);
+int launch_fuse_ring(Kern kern, const FuseParams& prm, size_t smem, cudaStream_t stream) {
     const DeviceInfo di = device_info();
     if (!di.ok || smem > 227 * 1024 || cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
         cudaGetLastError();
@@ -137,19 +137,6 @@ inline size_t lowres_plan(FuseParams& prm, int tile_pix, int chunk, int stages, 
         if (lr.hm[s] != lr.hm[0] || lr.wm[s] != lr.wm[0] || lr.ha[s] != lr.ha[0] || lr.wa[s] != lr.wa[0]) lr.same_geometry = 0;
     return sizeof(float) * (size_t)lr.stage_floats * stages + 2 * stages * sizeof(uint64_t) +
            fuse_tally_smem_bytes(prm.K, KT, nthreads, P) + 128;
-}
-
-template <int NCW, int P, typename Kern>
-int launch_fuse_lowres(Kern kern, const FuseParams& prm, size_t smem, cudaStream_t stream) {
-    const DeviceInfo di = device_info();
-    if (!di.ok || cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-        cudaGetLastError();
-        return MSPL_ERR_CUDA;
-    }
-    constexpr int TP = NCW * 32 * P;
-    const int64_t n_tiles = prm.n_img * ((prm.hw + TP - 1) / TP);
-    kern<<<(unsigned)(n_tiles < di.sms ? n_tiles : di.sms), (NCW + 1) * 32, smem, stream>>>(prm);
-    return launch_status();
 }
 
 }  // namespace mspl

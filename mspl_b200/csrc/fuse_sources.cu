@@ -6,51 +6,37 @@
 
 namespace mspl {
 
-// Build-time choice of the K1 variants (picked from the tools/k1_sweep measurements on B200, see profiles/).
-#ifndef MSPL_FUSE_CH
-#define MSPL_FUSE_CH 5        // classes per chunk: 13 -> 5+5+3, 20 -> 4x5, 5 -> one exact two-sweep chunk
-#endif
-#ifndef MSPL_FUSE_MINB
-#define MSPL_FUSE_MINB 2      // direct kernel: resident CTAs per SM the register allocator must leave room for
-#endif
-#ifndef MSPL_USE_TMA
-#define MSPL_USE_TMA 1
-#endif
-#ifndef MSPL_LOWRES_NCW
-#define MSPL_LOWRES_NCW 15     // K1-lowres: consumer warps (instruction-bound kernel; 16 warps split the register file evenly)
-#endif
-#ifndef MSPL_LOWRES_STAGES
-#define MSPL_LOWRES_STAGES 4
-#endif
-
 // TMA-staged kernel configuration <consumer warps, pixels per thread, classes per chunk, ring stages>, picked from the
 // tools/k1_sweep runs on B200 (profiles/): 15 consumer + 1 producer warps = 16 warps, so the register file splits evenly
 // (128 regs/thread); 960-pixel tiles, 4 x 38.4 KB stages.  Since round 2 every policy runs this one shape: with the classes
 // visited grouped by target the per-target maxima cost nothing extra per class (pixel_math.cuh), so 'half' / 'prob' differ
 // from 'all' only in the per-source epilogue.  More than 5 target classes: 3 stages (their histogram and group slots need
 // the shared memory of the fourth).
-template <int KT> struct TmaCfgFor { using type = TmaCfg<15, 2, MSPL_FUSE_CH, 4>; static constexpr int kStages = 4; };
-template <> struct TmaCfgFor<8> { using type = TmaCfg<15, 2, MSPL_FUSE_CH, 3>; static constexpr int kStages = 3; };
+template <int KT> constexpr int kTmaStages = KT <= 5 ? 4 : 3;
 constexpr int kDirectThreads = 256;
+constexpr int kDirectMinBlocks = 2;     // direct kernel without GK: resident CTAs per SM the register allocator must leave room for
+// K1-lowres: 15 consumer warps (instruction-bound kernel; 16 warps split the register file evenly), 4 ring stages
+constexpr int kLowresNcw = 15, kLowresStages = 4;
 
 template <int KT>
-static int dispatch_fuse(FuseParams& prm, bool aligned, bool gk, cudaStream_t stream) {
-    constexpr int CH = MSPL_FUSE_CH;
-    using Cfg = typename TmaCfgFor<KT>::type;
-    constexpr int NST = TmaCfgFor<KT>::kStages;
+static int dispatch_fuse(FuseParams& prm, bool gk, cudaStream_t stream) {
+    constexpr int CH = kFuseChunk, NST = kTmaStages<KT>;
+    using Cfg = TmaCfg<15, 2, CH, NST>;
     if (!build_class_order(prm, CH)) return MSPL_ERR_UNSUPPORTED;
-    if (MSPL_USE_TMA && aligned && tma_eligible(prm)) {
+    if (tma_eligible(prm)) {
+        const size_t smem = Cfg::smem_bytes(prm.K, KT);
         // nothing but hard labels requested under a vote policy (the reference's own generation loop): no softmax at all
         const bool labels_only = prm.policy == MSPL_POLICY_VOTE && !prm.conf && !prm.unc && !prm.conf_hist && !prm.marginal;
         bool any_kld = false;
         for (int s = 0; s < prm.S; ++s) any_kld = any_kld || prm.kld[s] != nullptr;
-        if (labels_only && !any_kld) return launch_fuse_tma<Cfg>(fuse_labels_tma_kernel<15, 2, CH, NST, KT>, prm, KT, stream);
-        if (gk) return launch_fuse_tma<Cfg>(fuse_sources_tma_kernel<15, 2, CH, NST, KT, true>, prm, KT, stream);
-        return launch_fuse_tma<Cfg>(fuse_sources_tma_kernel<15, 2, CH, NST, KT, false>, prm, KT, stream);
+        if (labels_only && !any_kld) return launch_fuse_ring<Cfg>(fuse_labels_tma_kernel<15, 2, CH, NST, KT>, prm, smem, stream);
+        if (gk) return launch_fuse_ring<Cfg>(fuse_sources_tma_kernel<15, 2, CH, NST, KT, true>, prm, smem, stream);
+        return launch_fuse_ring<Cfg>(fuse_sources_tma_kernel<15, 2, CH, NST, KT, false>, prm, smem, stream);
     }
     // odd shapes / unaligned views: per-thread scalar streaming loads, same math
     if (gk) return launch_fuse_direct<kDirectThreads>(fuse_sources_direct_kernel<CH, KT, true, kDirectThreads, 1>, prm, KT, stream);
-    return launch_fuse_direct<kDirectThreads>(fuse_sources_direct_kernel<CH, KT, false, kDirectThreads, MSPL_FUSE_MINB>, prm, KT, stream);
+    return launch_fuse_direct<kDirectThreads>(fuse_sources_direct_kernel<CH, KT, false, kDirectThreads, kDirectMinBlocks>, prm, KT,
+                                              stream);
 }
 
 // merge_outputs (uest_seg_multi_os.py:695-718) on (S, npix) hard labels.
@@ -62,13 +48,7 @@ __global__ void __launch_bounds__(256) vote_labels_kernel(const uint8_t* __restr
             const uint32_t l = labels[s * npix + i];
             if (l < (uint32_t)K) votes += 1u << (4 * l);   // values outside [0,K) match no class_id, as in the reference
         }
-        int bk = 0;
-        uint32_t bc = votes & 15u;
-        for (int k = 1; k < K; ++k) {
-            const uint32_t c = (votes >> (4 * k)) & 15u;
-            if (c > bc) { bc = c; bk = k; }
-        }
-        merged[i] = (uint8_t)(((int)bc < vote_t) ? ignore : bk);
+        merged[i] = (uint8_t)merge_votes<MSPL_MAX_CLASSES>(votes, vote_t, ignore);
     }
 }
 
@@ -80,8 +60,8 @@ extern "C" const char* mspl_fuse_variant(void) {
     static char name[256];
     snprintf(name, sizeof(name),
              "tma-bulk ring, CH=%d, classes visited grouped by target, packed f32x2 math: <15 consumer warps, P=2, 4 stages> for "
-             "every policy; direct-ldg P=1 fallback for unaligned shapes%s",
-             MSPL_FUSE_CH, MSPL_USE_TMA ? "" : " (TMA disabled at build time)");
+             "every policy; direct-ldg P=1 fallback for unaligned shapes",
+             kFuseChunk);
     return name;
 }
 
@@ -97,7 +77,7 @@ static int class_order_of_table(const uint8_t* lut, int num_classes, int num_tar
         if (lut[c] >= num_target_classes) return MSPL_ERR_BAD_ARG;
         prm.lut[0][c] = lut[c];
     }
-    return build_class_order(prm, MSPL_FUSE_CH) ? MSPL_OK : MSPL_ERR_UNSUPPORTED;
+    return build_class_order(prm, kFuseChunk) ? MSPL_OK : MSPL_ERR_UNSUPPORTED;
 }
 
 extern "C" int mspl_class_order(const uint8_t* lut, int num_classes, int num_target_classes, uint8_t* row, uint8_t* seg,
@@ -107,9 +87,9 @@ extern "C" int mspl_class_order(const uint8_t* lut, int num_classes, int num_tar
     const int rc = class_order_of_table(lut, num_classes, num_target_classes, prm);
     if (rc != MSPL_OK) return rc;
     memcpy(row, prm.order[0].row, (size_t)num_classes);
-    memcpy(seg, prm.order[0].seg, (size_t)((num_classes + MSPL_FUSE_CH - 1) / MSPL_FUSE_CH));
+    memcpy(seg, prm.order[0].seg, (size_t)((num_classes + kFuseChunk - 1) / kFuseChunk));
     *present = prm.order[0].present;
-    return MSPL_FUSE_CH;
+    return kFuseChunk;
 }
 
 extern "C" int mspl_class_order_votes(const uint8_t* lut, int num_classes, int num_target_classes, uint32_t* vote, uint32_t* nchunk) {
@@ -128,54 +108,78 @@ extern "C" int mspl_class_order_shape(const uint8_t* lut, int num_classes, int n
     return rc != MSPL_OK ? rc : (int)prm.order[0].shape;
 }
 
+// Checks and copies into prm what both K1 entry points take, returning MSPL_OK or the status the entry point returns.  With no
+// images (prm.n_img == 0) the sources are not looked at.  main_hw / aux_hw: K1-lowres's head sizes, nullptr at full resolution;
+// K1-lowres also needs 16-byte aligned logits, KLD maps, confidences and uncertainties and hw % 4 == 0.  The checks run in a
+// fixed order: of several bad arguments, the first one checked decides the status.
+static int fuse_args(FuseParams& prm, int S, const float* const* main_logits, const float* const* aux_logits, const int* num_classes,
+                     const uint8_t* const* lut, const int* main_hw, const int* aux_hw, int64_t num_images, int64_t hw, int K,
+                     int policy, int vote_t, int ignore_label, int ds_rate, uint8_t* label, float* conf, float* unc,
+                     float* const* kld_per_source, unsigned long long* class_hist, unsigned long long* conf_hist,
+                     unsigned long long* marginal_count) {
+    const bool lowres = main_hw != nullptr;
+    if (S < 1 || S > MSPL_MAX_SOURCES || K < 2 || K > MSPL_MAX_CLASSES) return MSPL_ERR_BAD_ARG;
+    if (!main_logits || !aux_logits || !num_classes || !lut || !label || !class_hist) return MSPL_ERR_BAD_ARG;
+    if (num_images < 0 || ds_rate < 1) return MSPL_ERR_BAD_ARG;
+    if (ignore_label < 0 || ignore_label >= K) return MSPL_ERR_BAD_ARG;
+    if (policy != MSPL_POLICY_VOTE && policy != MSPL_POLICY_PROB) return MSPL_ERR_BAD_ARG;
+    if (conf_hist && !conf) return MSPL_ERR_BAD_ARG;
+    memset(&prm, 0, sizeof(prm));
+    if (num_images == 0) return MSPL_OK;
+    if (lowres && hw % 4 != 0) return MSPL_ERR_UNSUPPORTED;
+    const size_t align = lowres ? 16 : 4;      // the direct kernel reads logits one float at a time
+    for (int s = 0; s < S; ++s) {
+        const int C = num_classes[s];
+        if (C < 1 || C > MSPL_MAX_SRC_CLASSES || !main_logits[s] || !aux_logits[s] || !lut[s]) return MSPL_ERR_BAD_ARG;
+        if (lowres) {
+            if (main_hw[2 * s] < 1 || main_hw[2 * s + 1] < 1 || aux_hw[2 * s] < 1 || aux_hw[2 * s + 1] < 1) return MSPL_ERR_BAD_ARG;
+            prm.lr.hm[s] = main_hw[2 * s]; prm.lr.wm[s] = main_hw[2 * s + 1];
+            prm.lr.ha[s] = aux_hw[2 * s]; prm.lr.wa[s] = aux_hw[2 * s + 1];
+        }
+        if (!aligned_to(main_logits[s], align) || !aligned_to(aux_logits[s], align)) return MSPL_ERR_ALIGN;
+        prm.main[s] = main_logits[s];
+        prm.aux[s] = aux_logits[s];
+        prm.kld[s] = kld_per_source ? kld_per_source[s] : nullptr;
+        if (lowres && prm.kld[s] && !aligned_to(prm.kld[s], 16)) return MSPL_ERR_ALIGN;
+        prm.C[s] = C;
+        for (int c = 0; c < C; ++c) {
+            if (lut[s][c] >= K) return MSPL_ERR_BAD_ARG;
+            prm.lut[s][c] = lut[s][c];
+        }
+    }
+    if ((lowres && !aligned_to(label, 4)) || (conf && !aligned_to(conf, align)) || (unc && !aligned_to(unc, align)))
+        return MSPL_ERR_ALIGN;
+    if (!aligned_to(class_hist, 8) || (conf_hist && !aligned_to(conf_hist, 8)) || (marginal_count && !aligned_to(marginal_count, 8)))
+        return MSPL_ERR_ALIGN;
+    prm.S = S; prm.K = K; prm.policy = policy; prm.vote_t = vote_t < 1 ? 1 : vote_t;
+    prm.ignore = ignore_label; prm.ds_rate = ds_rate;
+    prm.n_img = num_images; prm.hw = hw;
+    prm.label = label; prm.conf = conf; prm.unc = unc;
+    prm.class_hist = class_hist; prm.conf_hist = conf_hist; prm.marginal = marginal_count;
+    return MSPL_OK;
+}
+
+// Per-target-class probabilities are only needed when a pixel can win without every source's vote.
+// (under a vote policy they only ever feed conf, so a call without conf does not need them either)
+static bool needs_target_probs(const FuseParams& prm) {
+    return prm.policy == MSPL_POLICY_PROB || (prm.vote_t < prm.S && prm.conf != nullptr);
+}
+
 extern "C" int mspl_fuse_sources(int num_sources, const float* const* main_logits, const float* const* aux_logits,
                                  const int* num_classes, const uint8_t* const* lut, int64_t num_images,
                                  int64_t pixels_per_image, int num_target_classes, int policy, int vote_t,
                                  int ignore_label, int ds_rate, uint8_t* label, float* conf, float* unc,
                                  float* const* kld_per_source, unsigned long long* class_hist,
                                  unsigned long long* conf_hist, unsigned long long* marginal_count, void* stream) {
-    const int S = num_sources, K = num_target_classes;
-    if (S < 1 || S > MSPL_MAX_SOURCES || K < 2 || K > MSPL_MAX_CLASSES) return MSPL_ERR_BAD_ARG;
-    if (!main_logits || !aux_logits || !num_classes || !lut || !label || !class_hist) return MSPL_ERR_BAD_ARG;
-    if (num_images < 0 || pixels_per_image < 1 || ds_rate < 1) return MSPL_ERR_BAD_ARG;
-    if (ignore_label < 0 || ignore_label >= K) return MSPL_ERR_BAD_ARG;
-    if (policy != MSPL_POLICY_VOTE && policy != MSPL_POLICY_PROB) return MSPL_ERR_BAD_ARG;
-    if (conf_hist && !conf) return MSPL_ERR_BAD_ARG;
-    if (num_images == 0) return MSPL_OK;
-
+    if (pixels_per_image < 1) return MSPL_ERR_BAD_ARG;
     FuseParams prm;
-    memset(&prm, 0, sizeof(prm));
-    int P = (pixels_per_image % 4 == 0) ? 4 : 1;
-    for (int s = 0; s < S; ++s) {
-        const int C = num_classes[s];
-        if (C < 1 || C > MSPL_MAX_SRC_CLASSES || !main_logits[s] || !aux_logits[s] || !lut[s]) return MSPL_ERR_BAD_ARG;
-        if (!aligned_to(main_logits[s], 4) || !aligned_to(aux_logits[s], 4)) return MSPL_ERR_ALIGN;
-        prm.main[s] = main_logits[s];
-        prm.aux[s] = aux_logits[s];
-        prm.kld[s] = kld_per_source ? kld_per_source[s] : nullptr;
-        prm.C[s] = C;
-        for (int c = 0; c < C; ++c) {
-            if (lut[s][c] >= K) return MSPL_ERR_BAD_ARG;
-            prm.lut[s][c] = lut[s][c];
-        }
-        if (!aligned_to(prm.main[s], 16) || !aligned_to(prm.aux[s], 16) || (prm.kld[s] && !aligned_to(prm.kld[s], 16))) P = 1;
-    }
-    if (!aligned_to(label, 4) || (conf && !aligned_to(conf, 16)) || (unc && !aligned_to(unc, 16))) P = 1;
-    if ((conf && !aligned_to(conf, 4)) || (unc && !aligned_to(unc, 4))) return MSPL_ERR_ALIGN;
-    if (!aligned_to(class_hist, 8) || (conf_hist && !aligned_to(conf_hist, 8)) || (marginal_count && !aligned_to(marginal_count, 8)))
-        return MSPL_ERR_ALIGN;
-
-    prm.S = S; prm.K = K; prm.policy = policy; prm.vote_t = vote_t < 1 ? 1 : vote_t;
-    prm.ignore = ignore_label; prm.ds_rate = ds_rate;
-    prm.n_img = num_images; prm.hw = pixels_per_image;
-    prm.label = label; prm.conf = conf; prm.unc = unc;
-    prm.class_hist = class_hist; prm.conf_hist = conf_hist; prm.marginal = marginal_count;
-
-    // Per-target-class probabilities are only needed when a pixel can win without every source's vote.
-    // (under a vote policy they only ever feed conf, so a call without conf does not need them either)
-    const bool gk = (policy == MSPL_POLICY_PROB) || (prm.vote_t < S && conf != nullptr);
+    const int rc = fuse_args(prm, num_sources, main_logits, aux_logits, num_classes, lut, nullptr, nullptr, num_images,
+                             pixels_per_image, num_target_classes, policy, vote_t, ignore_label, ds_rate, label, conf, unc,
+                             kld_per_source, class_hist, conf_hist, marginal_count);
+    if (rc != MSPL_OK || prm.n_img == 0) return rc;
+    const bool gk = needs_target_probs(prm);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    return K <= 5 ? dispatch_fuse<5>(prm, P == 4, gk, st) : dispatch_fuse<8>(prm, P == 4, gk, st);
+    return prm.K <= 5 ? dispatch_fuse<5>(prm, gk, st) : dispatch_fuse<8>(prm, gk, st);
 }
 
 extern "C" int mspl_fuse_sources_lowres(int num_sources, const float* const* main_logits, const float* const* aux_logits,
@@ -184,69 +188,39 @@ extern "C" int mspl_fuse_sources_lowres(int num_sources, const float* const* mai
                                         int ignore_label, int ds_rate, uint8_t* label, float* conf, float* unc,
                                         float* const* kld_per_source, unsigned long long* class_hist,
                                         unsigned long long* conf_hist, unsigned long long* marginal_count, void* stream) {
-    const int S = num_sources, K = num_target_classes;
-    if (S < 1 || S > MSPL_MAX_SOURCES || K < 2 || K > MSPL_MAX_CLASSES) return MSPL_ERR_BAD_ARG;
-    if (!main_logits || !aux_logits || !num_classes || !lut || !main_hw || !aux_hw || !label || !class_hist) return MSPL_ERR_BAD_ARG;
-    if (num_images < 0 || out_h < 1 || out_w < 1 || ds_rate < 1) return MSPL_ERR_BAD_ARG;
-    if (ignore_label < 0 || ignore_label >= K) return MSPL_ERR_BAD_ARG;
-    if (policy != MSPL_POLICY_VOTE && policy != MSPL_POLICY_PROB) return MSPL_ERR_BAD_ARG;
-    if (conf_hist && !conf) return MSPL_ERR_BAD_ARG;
-    if (num_images == 0) return MSPL_OK;
+    if (!main_hw || !aux_hw || out_h < 1 || out_w < 1) return MSPL_ERR_BAD_ARG;
     FuseParams prm;
-    memset(&prm, 0, sizeof(prm));
-    const int64_t hw = (int64_t)out_h * out_w;
-    if (hw % 4 != 0) return MSPL_ERR_UNSUPPORTED;
-    for (int s = 0; s < S; ++s) {
-        const int C = num_classes[s];
-        if (C < 1 || C > MSPL_MAX_SRC_CLASSES || !main_logits[s] || !aux_logits[s] || !lut[s]) return MSPL_ERR_BAD_ARG;
-        if (main_hw[2 * s] < 1 || main_hw[2 * s + 1] < 1 || aux_hw[2 * s] < 1 || aux_hw[2 * s + 1] < 1) return MSPL_ERR_BAD_ARG;
-        if (!aligned_to(main_logits[s], 16) || !aligned_to(aux_logits[s], 16)) return MSPL_ERR_ALIGN;
-        prm.main[s] = main_logits[s];
-        prm.aux[s] = aux_logits[s];
-        prm.kld[s] = kld_per_source ? kld_per_source[s] : nullptr;
-        if (prm.kld[s] && !aligned_to(prm.kld[s], 16)) return MSPL_ERR_ALIGN;
-        prm.C[s] = C;
-        prm.lr.hm[s] = main_hw[2 * s]; prm.lr.wm[s] = main_hw[2 * s + 1];
-        prm.lr.ha[s] = aux_hw[2 * s]; prm.lr.wa[s] = aux_hw[2 * s + 1];
-        for (int c = 0; c < C; ++c) {
-            if (lut[s][c] >= K) return MSPL_ERR_BAD_ARG;
-            prm.lut[s][c] = lut[s][c];
-        }
-    }
-    if (!aligned_to(label, 4) || (conf && !aligned_to(conf, 16)) || (unc && !aligned_to(unc, 16))) return MSPL_ERR_ALIGN;
-    if (!aligned_to(class_hist, 8) || (conf_hist && !aligned_to(conf_hist, 8)) || (marginal_count && !aligned_to(marginal_count, 8)))
-        return MSPL_ERR_ALIGN;
-    prm.S = S; prm.K = K; prm.policy = policy; prm.vote_t = vote_t < 1 ? 1 : vote_t;
-    prm.ignore = ignore_label; prm.ds_rate = ds_rate;
-    prm.n_img = num_images; prm.hw = hw;
+    const int rc = fuse_args(prm, num_sources, main_logits, aux_logits, num_classes, lut, main_hw, aux_hw, num_images,
+                             (int64_t)out_h * out_w, num_target_classes, policy, vote_t, ignore_label, ds_rate, label, conf, unc,
+                             kld_per_source, class_hist, conf_hist, marginal_count);
+    if (rc != MSPL_OK || prm.n_img == 0) return rc;
     prm.lr.H = out_h; prm.lr.W = out_w;
-    prm.label = label; prm.conf = conf; prm.unc = unc;
-    prm.class_hist = class_hist; prm.conf_hist = conf_hist; prm.marginal = marginal_count;
 
-    constexpr int NCW = MSPL_LOWRES_NCW, P = 2, CH = MSPL_FUSE_CH, NST = MSPL_LOWRES_STAGES;
-    constexpr int kThreads = (NCW + 1) * 32;
-    const bool gk = (policy == MSPL_POLICY_PROB) || (prm.vote_t < S && conf != nullptr);
+    constexpr int NCW = kLowresNcw, P = 2, CH = kFuseChunk, NST = kLowresStages;
+    using Cfg = TmaCfg<NCW, P, CH, NST>;
+    const bool gk = needs_target_probs(prm);
+    const int K = prm.K;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (!build_class_order(prm, CH)) return MSPL_ERR_UNSUPPORTED;
     if (K <= 5) {   // common geometries (e.g. ESPDNetUE at 480x256: 3 rows x 240 / 3 rows x 120 floats per class) fit fixed class
                     // strides, which turn every interpolation tap into an immediate-offset shared-memory load
         constexpr int MS = 768, AS = 384;
         FuseParams fixed = prm;
-        const size_t fsmem = lowres_plan(fixed, NCW * 32 * P, CH, NST, 5, kThreads, P, MS, AS);
+        const size_t fsmem = lowres_plan(fixed, Cfg::kTilePix, CH, NST, 5, Cfg::kThreads, P, MS, AS);
         if (fsmem != 0 && fsmem <= 227 * 1024) {
-            if (gk) return launch_fuse_lowres<NCW, P>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 5, true, MS, AS>, fixed, fsmem, st);
-            return launch_fuse_lowres<NCW, P>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 5, false, MS, AS>, fixed, fsmem, st);
+            if (gk) return launch_fuse_ring<Cfg>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 5, true, MS, AS>, fixed, fsmem, st);
+            return launch_fuse_ring<Cfg>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 5, false, MS, AS>, fixed, fsmem, st);
         }
     }
     const int KT = K <= 5 ? 5 : 8;
-    const size_t smem = lowres_plan(prm, NCW * 32 * P, CH, NST, KT, kThreads, P);
+    const size_t smem = lowres_plan(prm, Cfg::kTilePix, CH, NST, KT, Cfg::kThreads, P);
     if (smem == 0 || smem > 227 * 1024) return MSPL_ERR_UNSUPPORTED;    // caller upsamples and uses mspl_fuse_sources instead
     if (K <= 5) {
-        if (gk) return launch_fuse_lowres<NCW, P>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 5, true>, prm, smem, st);
-        return launch_fuse_lowres<NCW, P>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 5, false>, prm, smem, st);
+        if (gk) return launch_fuse_ring<Cfg>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 5, true>, prm, smem, st);
+        return launch_fuse_ring<Cfg>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 5, false>, prm, smem, st);
     }
-    if (gk) return launch_fuse_lowres<NCW, P>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 8, true>, prm, smem, st);
-    return launch_fuse_lowres<NCW, P>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 8, false>, prm, smem, st);
+    if (gk) return launch_fuse_ring<Cfg>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 8, true>, prm, smem, st);
+    return launch_fuse_ring<Cfg>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 8, false>, prm, smem, st);
 }
 
 extern "C" int mspl_vote_labels(const uint8_t* labels, int num_sources, int64_t num_pixels, int num_target_classes,

@@ -180,11 +180,13 @@ struct ClassOrder {
 
 // ---- compiled chunk shapes ---------------------------------------------------------------------------------------------
 // Everything the chunk loop does per source follows from (C, nchunk, seg[0..nchunk)) alone.  The shapes of the greenhouse
-// tables (data_loader/segmentation/greenhouse.py SOURCE_TABLES, at kShapeChunk classes per chunk) are listed here, and the
+// tables (data_loader/segmentation/greenhouse.py SOURCE_TABLES, at kFuseChunk classes per chunk) are listed here, and the
 // TMA kernel runs a fully unrolled body for each of them: group commits only where a group ends, no rescale on the first chunk,
 // and a tail chunk that loads and folds only its real classes (so the producer writes no padding for it).  Any other shape
 // runs the generic loop.  build_class_order sets ClassOrder::shape.
-constexpr int kShapeChunk = 5;
+// kFuseChunk is the chunk size of every K1 kernel the library launches (classes per chunk: 13 -> 5+5+3, 20 -> 4x5, 5 -> one
+// exact two-sweep chunk, picked from the tools/k1_sweep measurements on B200, see profiles/).
+constexpr int kFuseChunk = 5;
 constexpr int kMaxShapeChunks = 4;
 struct SourceShape {
     int C, nchunk;
@@ -295,10 +297,7 @@ constexpr float kMaxSharedExpGap = 16.f;
 // ~1.5 ulp(z) in the exponent: at most 7.6e-6 relative up to |Mz| = 48 (|Rz| <= 64), but 3e-5 at |z| = 256.  Beyond 48 the
 // slow path recomputes the reference's own expression e^{z_c - Mz} from the rounded z.  (A limit of 32 put ~3 pixels in 10^5
 // of the benchmark's N(0, 6.4^2) fused logits on the slow path and cost K1 1.6 %; 48 is 7.5 sigma away.)
-#ifndef MSPL_MAX_EXP_LOGIT
-#define MSPL_MAX_EXP_LOGIT 48.f
-#endif
-constexpr float kMaxSharedExpLogit = MSPL_MAX_EXP_LOGIT;
+constexpr float kMaxSharedExpLogit = 48.f;
 
 // Mz: the maximum of the source's fused logits, per pixel.
 template <int P>

@@ -134,6 +134,44 @@ def test_class_order_groups_classes_by_target(lib):
     assert lib.mspl_class_order_votes(bad, 3, 5, (ctypes.c_uint32 * 8)(), ctypes.byref(ctypes.c_uint32())) == -1
 
 
+def _fuse_status(lib, lowres, S=3, C=13, K=5, policy=0, ignore=4, ds_rate=1, conf=True, conf_hist=True, bad_entry=False,
+                 misaligned=False, head=(64, 120), out=(256, 480)):
+    """Status of one K1 entry point call whose device pointers are fake: the argument checks only test their alignment, so
+    every call below has to return before any CUDA work (a call that got as far as a launch would report a CUDA error)."""
+    import ctypes
+    vp, n = ctypes.c_void_p, 9
+    fake = 1 << 32
+    main = (vp * n)(*[fake + (s << 24) + (2 if misaligned and s == 0 else 0) for s in range(n)])
+    aux = (vp * n)(*[fake + ((n + s) << 24) for s in range(n)])
+    ncls = (ctypes.c_int * n)(*[C] * n)
+    tables = [(ctypes.c_ubyte * 256)(*[c % 5 for c in range(256)]) for _ in range(n)]
+    if bad_entry:
+        tables[1][2] = K
+    lut = (vp * n)(*[ctypes.addressof(t) for t in tables])
+    label, conf_p, unc, class_hist, hist = (fake + (i << 28) for i in range(1, 6))
+    common = [K, policy, 2, ignore, ds_rate, label, conf_p if conf else None, unc, None, class_hist,
+              hist if conf_hist else None, None, None]
+    if lowres:
+        main_hw = (ctypes.c_int * (2 * n))(*[2 * v for v in head] * n)
+        aux_hw = (ctypes.c_int * (2 * n))(*list(head) * n)
+        return lib.mspl_fuse_sources_lowres(S, main, aux, ncls, lut, main_hw, aux_hw, 1, out[0], out[1], *common)
+    return lib.mspl_fuse_sources(S, main, aux, ncls, lut, 1, out[0] * out[1], *common)
+
+
+@pytest.mark.parametrize("lowres", [False, True])
+def test_fuse_entry_points_reject_bad_arguments(lib, lowres):
+    """Argument checks of mspl_fuse_sources and mspl_fuse_sources_lowres, one invalid argument per call (no GPU).  One image
+    throughout: a call without images returns MSPL_OK before the per-source checks."""
+    BAD, ALIGN, UNSUPPORTED = -1, -2, -3
+    cases = [(dict(S=0), BAD), (dict(S=9), BAD), (dict(K=1), BAD), (dict(K=9), BAD), (dict(policy=2), BAD),
+             (dict(ignore=5), BAD), (dict(conf=False), BAD), (dict(C=0), BAD), (dict(C=257), BAD),
+             (dict(bad_entry=True), BAD), (dict(ds_rate=0), BAD), (dict(misaligned=True), ALIGN)]
+    if lowres:
+        cases += [(dict(head=(0, 120)), BAD), (dict(head=(64, 0)), BAD), (dict(out=(3, 5)), UNSUPPORTED)]
+    for kw, want in cases:
+        assert _fuse_status(lib, lowres, **kw) == want, kw
+
+
 def test_vote_threshold_follows_merge_outputs_rule():
     """merge_outputs' threshold rule (uest_seg_multi_os.py:697-705): None / 'half' / anything else -> S//2+1, 'all' -> S, an int
     (bool included, as `isinstance(thresh, int)` accepts it) <= S -> itself."""

@@ -24,7 +24,7 @@ from gpu_launch_probe import (KLD_ATOL, RTOL, _check_fusion, _oracle_settings, _
 
 pytestmark = pytest.mark.gpu
 
-CH = 5                              # MSPL_FUSE_CH: source classes per ring stage
+CH = 5                              # kFuseChunk: source classes per ring stage
 TILE = 960                          # pixels per tile of the TMA and lowres kernels (15 consumer warps x 32 lanes x 2 pixels)
 LEAN = dict(want_conf=False, want_unc=False, want_conf_hist=False, count_marginal=False)     # -> the labels-only kernel
 LOWRES_TOL = dict(conf_rtol=1e-4, conf_atol=1e-6, unc_rtol=1e-4, unc_atol=1e-5)             # test_fuse_sources_lowres's parity

@@ -110,7 +110,7 @@ static void run_variant(const char* name, Bench& b, F launch) {
         build_class_order(b.prm, CH);                                                                                            \
         if (tma_eligible(b.prm) && Cfg::smem_bytes(5, 5) <= 227 * 1024)                                                          \
             run_variant("tma ncw=" #NCW " P=" #P " CH=" #CH " stages=" #NST " gk=" #GK, b, [&] {                               \
-                return launch_fuse_tma<Cfg>(fuse_sources_tma_kernel<NCW, P, CH, NST, 5, GK>, b.prm, 5, 0);                       \
+                return launch_fuse_ring<Cfg>(fuse_sources_tma_kernel<NCW, P, CH, NST, 5, GK>, b.prm, Cfg::smem_bytes(5, 5), 0); \
             });                                                                                                                  \
         else printf("tma ncw=" #NCW " P=" #P " CH=" #CH " stages=" #NST ": not eligible / smem %zu\n", Cfg::smem_bytes(5, 5));  \
     }
@@ -122,7 +122,7 @@ static void run_variant(const char* name, Bench& b, F launch) {
         q.conf = nullptr; q.unc = nullptr; q.conf_hist = nullptr; q.marginal = nullptr;                                         \
         build_class_order(q, CH);                                                                                                \
         run_variant("labels-only ncw=" #NCW " P=" #P " CH=" #CH " stages=" #NST " (no softmax: z, arg-max, table, vote)", b, [&] { \
-            return launch_fuse_tma<Cfg>(fuse_labels_tma_kernel<NCW, P, CH, NST, 5>, q, 5, 0);                                    \
+            return launch_fuse_ring<Cfg>(fuse_labels_tma_kernel<NCW, P, CH, NST, 5>, q, Cfg::smem_bytes(5, 5), 0);              \
         });                                                                                                                      \
     }
 
@@ -133,7 +133,8 @@ static void run_variant(const char* name, Bench& b, F launch) {
         const size_t smem = lowres_plan(q, NCW * 32 * P, CH, NST, 5, (NCW + 1) * 32, P, 768, 384);                               \
         if (smem && smem <= 227 * 1024)                                                                                          \
             run_variant("lowres ncw=" #NCW " P=" #P " CH=" #CH " stages=" #NST " gk=" #GK, b, [&] {                            \
-                return launch_fuse_lowres<NCW, P>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 5, GK, 768, 384>, q, smem, 0);     \
+                return launch_fuse_ring<TmaCfg<NCW, P, CH, NST>>(fuse_sources_lowres_kernel<NCW, P, CH, NST, 5, GK, 768, 384>, q, \
+                                                                 smem, 0);                                               \
             });                                                                                                                  \
         else printf("lowres ncw=" #NCW " stages=" #NST ": smem %zu does not fit\n", smem);                                     \
     }
