@@ -245,6 +245,19 @@ MSPL_API int mspl_uw_ce_step(const float* main_logits, const float* aux_logits, 
                     const float* class_weights, int64_t num_images, int num_classes, int64_t pixels_per_image,
                     float alpha, double norm_pixels, float grad_scale, float* out3, float* d_main, float* d_aux,
                     unsigned long long* iou_counts, void* workspace, size_t workspace_bytes, void* stream);
+/* mspl_uw_ce_step on fp16 or bf16 logits (what a model run under autocast produces): logit_dtype is MSPL_DTYPE_F16 or
+ * MSPL_DTYPE_BF16, main_logits / aux_logits point to that type and d_main / d_aux receive the gradients in it.  The logits are
+ * upcast to fp32 (exact) and every per-pixel operation is the fp32 one; the IoU counts are those of the fp32 entry on the
+ * upcast logits; out3 stays f32.  The gradients are those of `loss * grad_scale * *grad_scale_dev` (grad_scale_dev: a device
+ * f32 scalar, NULL = 1), scaled before they are rounded to nearest even: a GradScaler's loss scale passed here keeps terms
+ * that would round to zero in fp16 unscaled.  Logit and gradient pointers must be 2-byte aligned (MSPL_ERR_ALIGN). */
+#define MSPL_DTYPE_F16 1
+#define MSPL_DTYPE_BF16 2
+MSPL_API int mspl_uw_ce_step_half(const void* main_logits, const void* aux_logits, int logit_dtype, const void* target,
+                         int target_is_u8, const float* class_weights, int64_t num_images, int num_classes,
+                         int64_t pixels_per_image, float alpha, double norm_pixels, float grad_scale,
+                         const float* grad_scale_dev, float* out3, void* d_main, void* d_aux,
+                         unsigned long long* iou_counts, void* workspace, size_t workspace_bytes, void* stream);
 /* K4-lowres (next-row component, SURVEY.md 8f-1): the same loss on the tensors ESPDNetUE hands to its closing
  * F.interpolate(..., size=(out_h,out_w), mode='bilinear', align_corners=True) calls (model/segmentation/espdnet_ue.py:301-302):
  * main_lowres (num_images, K, main_h, main_w), aux_lowres (num_images, K, aux_h, aux_w), target (num_images, out_h, out_w).

@@ -44,6 +44,8 @@ SIGNATURES = {
                                       c_vp, c_vp, c_sz, c_vp]),
     "mspl_uw_ce_step": (c_int, [c_vp, c_vp, c_vp, c_int, c_vp, c_i64, c_int, c_i64, c_f32, c_f64, c_f32, c_vp, c_vp, c_vp, c_vp,
                                 c_vp, c_sz, c_vp]),
+    "mspl_uw_ce_step_half": (c_int, [c_vp, c_vp, c_int, c_vp, c_int, c_vp, c_i64, c_int, c_i64, c_f32, c_f64, c_f32, c_vp, c_vp,
+                                     c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "mspl_uw_ce_lowres_fwd_bwd_u8": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_f32,
                                              c_f64, c_f32, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "mspl_uw_ce_lowres_fwd_bwd": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_f32, c_f64,

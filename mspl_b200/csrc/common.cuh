@@ -1,6 +1,8 @@
 // Shared device/host helpers for the mspl_b200 kernels (sm_100a).
 #pragma once
 #include <cuda_runtime.h>
+#include <cuda_fp16.h>
+#include <cuda_bf16.h>
 #include <stdint.h>
 #include <math.h>
 #include <initializer_list>
@@ -41,6 +43,49 @@ template <> struct PixVec<4> {
         __stcs(reinterpret_cast<float4*>(p), make_float4(v[0], v[1], v[2], v[3]));
     }
 };
+
+// ---- the same for fp16 / bf16 planes (autocast logits): loads upcast to fp32, which is exact; stores round to nearest even
+template <typename LT> MSPL_DEVINL float half_to_float(uint32_t bits);
+template <> MSPL_DEVINL float half_to_float<__half>(uint32_t bits) { return __half2float(__ushort_as_half((unsigned short)bits)); }
+template <> MSPL_DEVINL float half_to_float<__nv_bfloat16>(uint32_t bits) { return __uint_as_float(bits << 16); }
+template <typename LT> MSPL_DEVINL uint32_t float_to_half(float f);
+template <> MSPL_DEVINL uint32_t float_to_half<__half>(float f) { return __half_as_ushort(__float2half_rn(f)); }
+template <> MSPL_DEVINL uint32_t float_to_half<__nv_bfloat16>(float f) { return __bfloat16_as_ushort(__float2bfloat16_rn(f)); }
+
+// P consecutive 2-byte pixels of one class plane, P in {1, 2, 4}: one 2-, 4- or 8-byte access.
+template <typename LT, int P> struct HalfVec {
+    static MSPL_DEVINL void load(const LT* p, float (&v)[P]) {
+        uint32_t w[(P + 1) / 2];
+        if (P == 1) {
+            unsigned short b;
+            asm volatile("ld.global.nc.L1::no_allocate.b16 %0, [%1];" : "=h"(b) : "l"(p));
+            w[0] = b;
+        } else if (P == 2) {
+            asm volatile("ld.global.nc.L1::no_allocate.b32 %0, [%1];" : "=r"(w[0]) : "l"(p));
+        } else {
+            asm volatile("ld.global.nc.L1::no_allocate.v2.b32 {%0,%1}, [%2];" : "=r"(w[0]), "=r"(w[P > 2 ? 1 : 0]) : "l"(p));
+        }
+#pragma unroll
+        for (int i = 0; i < P; ++i) v[i] = half_to_float<LT>((w[i / 2] >> (16 * (i & 1))) & 0xffffu);
+    }
+    static MSPL_DEVINL void store(LT* p, const float (&v)[P]) {
+        uint32_t w[(P + 1) / 2];
+#pragma unroll
+        for (int i = 0; i < (P + 1) / 2; ++i)
+            w[i] = float_to_half<LT>(v[2 * i]) | (2 * i + 1 < P ? float_to_half<LT>(v[(2 * i + 1) % P]) << 16 : 0u);
+        if (P == 1) {
+            asm volatile("st.global.cs.b16 [%0], %1;" ::"l"(p), "h"((unsigned short)w[0]) : "memory");
+        } else if (P == 2) {
+            asm volatile("st.global.cs.b32 [%0], %1;" ::"l"(p), "r"(w[0]) : "memory");
+        } else {
+            asm volatile("st.global.cs.v2.b32 [%0], {%1,%2};" ::"l"(p), "r"(w[0]), "r"(w[P > 2 ? 1 : 0]) : "memory");
+        }
+    }
+};
+
+// Logit planes of element type LT: fp32 through PixVec, fp16 / bf16 through HalfVec.
+template <typename LT, int P> struct LogitVec : HalfVec<LT, P> {};
+template <int P> struct LogitVec<float, P> : PixVec<P> {};
 
 template <int P> MSPL_DEVINL void store_labels(uint8_t* p, const int (&l)[P]);
 template <> MSPL_DEVINL void store_labels<1>(uint8_t* p, const int (&l)[1]) { p[0] = (uint8_t)l[0]; }

@@ -205,13 +205,13 @@ MSPL_DEVINL void iou_flush(uint32_t* my_cnt, uint32_t* s_iou) {
 #ifndef MSPL_UWCE_BWD_P
 #define MSPL_UWCE_BWD_P 2
 #endif
-template <int P, int K, bool BWD, typename TT, bool IOU>
-__global__ void __launch_bounds__(kLossThreads, (K <= 6 ? MSPL_UWCE_MINB : 2)) uw_ce_fused_kernel(const float* __restrict__ main_l, const float* __restrict__ aux_l,
-                                                                   const TT* __restrict__ target, const float* __restrict__ cw,
-                                                                   int64_t n_img, int64_t hw, float alpha, double inv_n, float gscale,
-                                                                   float* __restrict__ out3, float* __restrict__ d_main,
-                                                                   float* __restrict__ d_aux, LossWorkspace* ws,
-                                                                   unsigned long long* __restrict__ iou_counts) {
+// The body of K4.  LT: logit and gradient element type, float or the __half / __nv_bfloat16 logits of an autocast forward;
+// every per-pixel operation is on the fp32 values either way.
+template <int P, int K, bool BWD, typename TT, bool IOU, typename LT>
+MSPL_DEVINL void uw_ce_fused(const LT* __restrict__ main_l, const LT* __restrict__ aux_l, const TT* __restrict__ target,
+                             const float* __restrict__ cw, int64_t n_img, int64_t hw, float alpha, double inv_n, float gscale,
+                             float* __restrict__ out3, LT* __restrict__ d_main, LT* __restrict__ d_aux, LossWorkspace* ws,
+                             unsigned long long* __restrict__ iou_counts) {
     __shared__ float s_w[K];
     __shared__ uint32_t s_iou[3 * K];
     __shared__ uint32_t s_cnt[IOU ? K * kLossThreads : 1];
@@ -233,9 +233,9 @@ __global__ void __launch_bounds__(kLossThreads, (K <= 6 ? MSPL_UWCE_MINB : 2)) u
         float m[K][P], a[K][P];
         long long t[P];
 #pragma unroll
-        for (int k = 0; k < K; ++k) PixVec<P>::load(main_l + base + k * hw, m[k]);
+        for (int k = 0; k < K; ++k) LogitVec<LT, P>::load(main_l + base + k * hw, m[k]);
 #pragma unroll
-        for (int k = 0; k < K; ++k) PixVec<P>::load(aux_l + base + k * hw, a[k]);
+        for (int k = 0; k < K; ++k) LogitVec<LT, P>::load(aux_l + base + k * hw, a[k]);
         load_targets<P>(target + n * hw + off, t);
         float gm[K][P], ga[K][P];
         float ce_sum = 0.f, d_sum = 0.f;
@@ -257,9 +257,9 @@ __global__ void __launch_bounds__(kLossThreads, (K <= 6 ? MSPL_UWCE_MINB : 2)) u
         acc_d += (double)d_sum;
         if (BWD) {
 #pragma unroll
-            for (int k = 0; k < K; ++k) PixVec<P>::store(d_main + base + k * hw, gm[k]);
+            for (int k = 0; k < K; ++k) LogitVec<LT, P>::store(d_main + base + k * hw, gm[k]);
 #pragma unroll
-            for (int k = 0; k < K; ++k) PixVec<P>::store(d_aux + base + k * hw, ga[k]);
+            for (int k = 0; k < K; ++k) LogitVec<LT, P>::store(d_aux + base + k * hw, ga[k]);
         }
         if (IOU) {
             iou_pixels += P;
@@ -275,6 +275,33 @@ __global__ void __launch_bounds__(kLossThreads, (K <= 6 ? MSPL_UWCE_MINB : 2)) u
         if (threadIdx.x < 3 * K && s_iou[threadIdx.x]) atomicAdd(iou_counts + threadIdx.x, (unsigned long long)s_iou[threadIdx.x]);
     }
     finish_loss<3>(acc_ce, acc_d, ws, inv_n, alpha, out3);
+}
+
+template <int P, int K, bool BWD, typename TT, bool IOU>
+__global__ void __launch_bounds__(kLossThreads, (K <= 6 ? MSPL_UWCE_MINB : 2)) uw_ce_fused_kernel(const float* __restrict__ main_l, const float* __restrict__ aux_l,
+                                                                   const TT* __restrict__ target, const float* __restrict__ cw,
+                                                                   int64_t n_img, int64_t hw, float alpha, double inv_n, float gscale,
+                                                                   float* __restrict__ out3, float* __restrict__ d_main,
+                                                                   float* __restrict__ d_aux, LossWorkspace* ws,
+                                                                   unsigned long long* __restrict__ iou_counts) {
+    uw_ce_fused<P, K, BWD, TT, IOU, float>(main_l, aux_l, target, cw, n_img, hw, alpha, inv_n, gscale, out3, d_main, d_aux, ws,
+                                           iou_counts);
+}
+
+// K4 on fp16 / bf16 logits.  gscale_dev (may be NULL): a device scalar the gradients are also scaled by -- the upstream
+// gradient of the autograd backward (a GradScaler's loss scale) -- applied BEFORE the rounding to LT, since gradient terms
+// far below the fp16 subnormal range only become representable after it.
+template <int P, int K, bool BWD, typename TT, bool IOU, typename LT>
+__global__ void __launch_bounds__(kLossThreads, (K <= 6 ? MSPL_UWCE_MINB : 2)) uw_ce_fused_half_kernel(const LT* __restrict__ main_l, const LT* __restrict__ aux_l,
+                                                                   const TT* __restrict__ target, const float* __restrict__ cw,
+                                                                   int64_t n_img, int64_t hw, float alpha, double inv_n, float gscale,
+                                                                   float* __restrict__ out3, LT* __restrict__ d_main,
+                                                                   LT* __restrict__ d_aux, LossWorkspace* ws,
+                                                                   unsigned long long* __restrict__ iou_counts,
+                                                                   const float* __restrict__ gscale_dev) {
+    if (BWD && gscale_dev) gscale *= __ldg(gscale_dev);
+    uw_ce_fused<P, K, BWD, TT, IOU, LT>(main_l, aux_l, target, cw, n_img, hw, alpha, inv_n, gscale, out3, d_main, d_aux, ws,
+                                        iou_counts);
 }
 
 }  // namespace mspl
@@ -663,19 +690,35 @@ static int64_t resident_grid(Kern kern, int64_t n_groups) {
     return blocks < 1 ? 1 : (blocks < cap ? blocks : cap);
 }
 
-template <int K, typename TT, bool IOU>
-static int launch_uw_ce(int P, bool bwd, const float* m, const float* a, const TT* t, const float* cw, int64_t n, int64_t hw,
-                        float alpha, double inv_n, float gs, float* out3, float* dm, float* da, LossWorkspace* ws,
+// Pixels per thread of the vector path for fp16 / bf16 logits (profiles/r05_loss_half_variants.txt).  Needs hw % P == 0 and
+// every plane 2P-byte aligned; otherwise P = 1.
+constexpr int kHalfFwdP = 4;
+constexpr int kHalfBwdP = 2;
+template <typename LT> constexpr int vec_pixels(bool bwd) {
+    return sizeof(LT) == 4 ? (bwd ? MSPL_UWCE_BWD_P : 4) : (bwd ? kHalfBwdP : kHalfFwdP);
+}
+
+template <int K, typename TT, bool IOU, typename LT>
+static int launch_uw_ce(bool vec, bool bwd, const LT* m, const LT* a, const TT* t, const float* cw, int64_t n, int64_t hw,
+                        float alpha, double inv_n, float gs, const float* gs_dev, float* out3, LT* dm, LT* da, LossWorkspace* ws,
                         unsigned long long* iou, cudaStream_t st) {
-    const int pv = P == 4 ? (bwd ? MSPL_UWCE_BWD_P : 4) : 1;
+    constexpr int PF = vec_pixels<LT>(false), PB = vec_pixels<LT>(true);
+    const int pv = vec ? (bwd ? PB : PF) : 1;
     const int64_t n_groups = n * (hw / pv);
 #define MSPL_UWCE(PP, BB)                                                                                                  \
     {                                                                                                                      \
-        auto kern = uw_ce_fused_kernel<PP, K, BB, TT, IOU>;                                                                        \
-        kern<<<(unsigned)resident_grid(kern, n_groups), kLossThreads, 0, st>>>(m, a, t, cw, n, hw, alpha, inv_n, gs, out3, dm, da, ws, iou); \
+        if constexpr (sizeof(LT) == 4) {                                                                                   \
+            auto kern = uw_ce_fused_kernel<PP, K, BB, TT, IOU>;                                                            \
+            kern<<<(unsigned)resident_grid(kern, n_groups), kLossThreads, 0, st>>>(m, a, t, cw, n, hw, alpha, inv_n, gs, out3, dm, da, \
+                                                                                   ws, iou);                                \
+        } else {                                                                                                           \
+            auto kern = uw_ce_fused_half_kernel<PP, K, BB, TT, IOU, LT>;                                                   \
+            kern<<<(unsigned)resident_grid(kern, n_groups), kLossThreads, 0, st>>>(m, a, t, cw, n, hw, alpha, inv_n, gs, out3, dm, da, \
+                                                                                   ws, iou, gs_dev);                        \
+        }                                                                                                                  \
     }
-    if (pv == 4 && !bwd) MSPL_UWCE(4, false)
-    else if (pv == MSPL_UWCE_BWD_P && bwd) MSPL_UWCE(MSPL_UWCE_BWD_P, true)
+    if (vec && !bwd) MSPL_UWCE(PF, false)
+    else if (vec) MSPL_UWCE(PB, true)
     else if (bwd) MSPL_UWCE(1, true)
     else MSPL_UWCE(1, false)
 #undef MSPL_UWCE
@@ -688,34 +731,45 @@ using namespace mspl;
 
 extern "C" size_t mspl_uw_ce_workspace_bytes(void) { return sizeof(LossWorkspace); }
 
-template <typename TT>
-static int uw_ce_entry(const float* main_logits, const float* aux_logits, const TT* target, const float* class_weights,
+template <typename TT, typename LT>
+static int uw_ce_entry(const LT* main_logits, const LT* aux_logits, const TT* target, const float* class_weights,
                        int64_t num_images, int num_classes, int64_t pixels_per_image, float alpha, double norm_pixels,
-                       float grad_scale, float* out3, float* d_main, float* d_aux, void* workspace, size_t workspace_bytes,
-                       unsigned long long* iou_counts, void* stream) {
+                       float grad_scale, const float* grad_scale_dev, float* out3, LT* d_main, LT* d_aux, void* workspace,
+                       size_t workspace_bytes, unsigned long long* iou_counts, void* stream) {
     if (!main_logits || !aux_logits || !target || !class_weights || !out3 || !workspace) return MSPL_ERR_BAD_ARG;
     if (!aligned_to(iou_counts, 8)) return MSPL_ERR_ALIGN;
     if ((d_main == nullptr) != (d_aux == nullptr)) return MSPL_ERR_BAD_ARG;
     if (num_images < 1 || pixels_per_image < 1 || num_classes < 1 || !(norm_pixels > 0)) return MSPL_ERR_BAD_ARG;
     if (workspace_bytes < sizeof(LossWorkspace)) return MSPL_ERR_WORKSPACE;
     if (num_classes > MSPL_MAX_CLASSES) return MSPL_ERR_UNSUPPORTED;
-    if (!aligned_to(main_logits, 4) || !aligned_to(aux_logits, 4) || !aligned_to(target, sizeof(TT)) || !aligned_to(workspace, 8))
+    if (!aligned_to(main_logits, sizeof(LT)) || !aligned_to(aux_logits, sizeof(LT)) || !aligned_to(d_main, sizeof(LT)) ||
+        !aligned_to(d_aux, sizeof(LT)) || !aligned_to(target, sizeof(TT)) || !aligned_to(workspace, 8) ||
+        !aligned_to(grad_scale_dev, 4))
         return MSPL_ERR_ALIGN;
     const bool bwd = d_main != nullptr;
-    // widest group of pixels per thread: rows of logits 16-byte aligned, and the group's targets loadable as one vector
-    // (two 16-byte loads of int64, one 4-byte load of uint8; the backward takes half a group)
-    int P = pick_vec(pixels_per_image, {main_logits, aux_logits, d_main, d_aux}) == 4 && aligned_to(target, sizeof(TT) == 8 ? 16 : 4) ? 4 : 1;
+    bool vec;
+    if (sizeof(LT) == 4) {
+        // widest group of pixels per thread: rows of logits 16-byte aligned, and the group's targets loadable as one vector
+        // (two 16-byte loads of int64, one 4-byte load of uint8; the backward takes half a group)
+        vec = pick_vec(pixels_per_image, {main_logits, aux_logits, d_main, d_aux}) == 4 && aligned_to(target, sizeof(TT) == 8 ? 16 : 4);
+    } else {
+        // P 2-byte pixels per thread: P-pixel rows, every plane 2P-byte aligned, the targets as 16-byte (int64) or P-byte loads
+        const int P = vec_pixels<LT>(bwd);
+        vec = pixels_per_image % P == 0 && aligned_to(target, sizeof(TT) == 8 ? 16 : P);
+        for (const void* q : {(const void*)main_logits, (const void*)aux_logits, (const void*)d_main, (const void*)d_aux})
+            vec = vec && aligned_to(q, 2 * P);
+    }
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     LossWorkspace* ws = static_cast<LossWorkspace*>(workspace);
     const double inv_n = 1.0 / norm_pixels;
 #define MSPL_CASE(KK)                                                                                                            \
     case KK:                                                                                                                     \
-        return iou_counts ? launch_uw_ce<KK, TT, true>(P, bwd, main_logits, aux_logits, target, class_weights, num_images,        \
-                                                       pixels_per_image, alpha, inv_n, grad_scale, out3, d_main, d_aux, ws,       \
-                                                       iou_counts, st)                                                            \
-                          : launch_uw_ce<KK, TT, false>(P, bwd, main_logits, aux_logits, target, class_weights, num_images,       \
-                                                        pixels_per_image, alpha, inv_n, grad_scale, out3, d_main, d_aux, ws,      \
-                                                        nullptr, st)
+        return iou_counts ? launch_uw_ce<KK, TT, true>(vec, bwd, main_logits, aux_logits, target, class_weights, num_images,      \
+                                                       pixels_per_image, alpha, inv_n, grad_scale, grad_scale_dev, out3, d_main,  \
+                                                       d_aux, ws, iou_counts, st)                                                 \
+                          : launch_uw_ce<KK, TT, false>(vec, bwd, main_logits, aux_logits, target, class_weights, num_images,     \
+                                                        pixels_per_image, alpha, inv_n, grad_scale, grad_scale_dev, out3, d_main, \
+                                                        d_aux, ws, nullptr, st)
     switch (num_classes) {
         MSPL_CASE(1); MSPL_CASE(2); MSPL_CASE(3); MSPL_CASE(4); MSPL_CASE(5); MSPL_CASE(6); MSPL_CASE(7); MSPL_CASE(8);
     }
@@ -728,7 +782,7 @@ extern "C" int mspl_uw_ce_fwd_bwd(const float* main_logits, const float* aux_log
                                   float grad_scale, float* out3, float* d_main, float* d_aux, void* workspace, size_t workspace_bytes,
                                   void* stream) {
     return uw_ce_entry<int64_t>(main_logits, aux_logits, target, class_weights, num_images, num_classes, pixels_per_image, alpha,
-                                norm_pixels, grad_scale, out3, d_main, d_aux, workspace, workspace_bytes, nullptr, stream);
+                                norm_pixels, grad_scale, nullptr, out3, d_main, d_aux, workspace, workspace_bytes, nullptr, stream);
 }
 
 extern "C" int mspl_uw_ce_fwd_bwd_u8(const float* main_logits, const float* aux_logits, const uint8_t* target, const float* class_weights,
@@ -736,7 +790,7 @@ extern "C" int mspl_uw_ce_fwd_bwd_u8(const float* main_logits, const float* aux_
                                      float grad_scale, float* out3, float* d_main, float* d_aux, void* workspace,
                                      size_t workspace_bytes, void* stream) {
     return uw_ce_entry<uint8_t>(main_logits, aux_logits, target, class_weights, num_images, num_classes, pixels_per_image, alpha,
-                                norm_pixels, grad_scale, out3, d_main, d_aux, workspace, workspace_bytes, nullptr, stream);
+                                norm_pixels, grad_scale, nullptr, out3, d_main, d_aux, workspace, workspace_bytes, nullptr, stream);
 }
 
 extern "C" int mspl_uw_ce_step(const float* main_logits, const float* aux_logits, const void* target, int target_is_u8,
@@ -745,11 +799,33 @@ extern "C" int mspl_uw_ce_step(const float* main_logits, const float* aux_logits
                                unsigned long long* iou_counts, void* workspace, size_t workspace_bytes, void* stream) {
     if (target_is_u8)
         return uw_ce_entry<uint8_t>(main_logits, aux_logits, static_cast<const uint8_t*>(target), class_weights, num_images,
-                                    num_classes, pixels_per_image, alpha, norm_pixels, grad_scale, out3, d_main, d_aux, workspace,
-                                    workspace_bytes, iou_counts, stream);
+                                    num_classes, pixels_per_image, alpha, norm_pixels, grad_scale, nullptr, out3, d_main, d_aux,
+                                    workspace, workspace_bytes, iou_counts, stream);
     return uw_ce_entry<int64_t>(main_logits, aux_logits, static_cast<const int64_t*>(target), class_weights, num_images, num_classes,
-                                pixels_per_image, alpha, norm_pixels, grad_scale, out3, d_main, d_aux, workspace, workspace_bytes,
-                                iou_counts, stream);
+                                pixels_per_image, alpha, norm_pixels, grad_scale, nullptr, out3, d_main, d_aux, workspace,
+                                workspace_bytes, iou_counts, stream);
+}
+
+extern "C" int mspl_uw_ce_step_half(const void* main_logits, const void* aux_logits, int logit_dtype, const void* target,
+                                    int target_is_u8, const float* class_weights, int64_t num_images, int num_classes,
+                                    int64_t pixels_per_image, float alpha, double norm_pixels, float grad_scale,
+                                    const float* grad_scale_dev, float* out3, void* d_main, void* d_aux,
+                                    unsigned long long* iou_counts, void* workspace, size_t workspace_bytes, void* stream) {
+    auto run = [&](auto lt) {
+        using LT = decltype(lt);
+        const LT *m = static_cast<const LT*>(main_logits), *a = static_cast<const LT*>(aux_logits);
+        LT *dm = static_cast<LT*>(d_main), *da = static_cast<LT*>(d_aux);
+        if (target_is_u8)
+            return uw_ce_entry<uint8_t, LT>(m, a, static_cast<const uint8_t*>(target), class_weights, num_images, num_classes,
+                                            pixels_per_image, alpha, norm_pixels, grad_scale, grad_scale_dev, out3, dm, da,
+                                            workspace, workspace_bytes, iou_counts, stream);
+        return uw_ce_entry<int64_t, LT>(m, a, static_cast<const int64_t*>(target), class_weights, num_images, num_classes,
+                                        pixels_per_image, alpha, norm_pixels, grad_scale, grad_scale_dev, out3, dm, da, workspace,
+                                        workspace_bytes, iou_counts, stream);
+    };
+    if (logit_dtype == MSPL_DTYPE_F16) return run(__half());
+    if (logit_dtype == MSPL_DTYPE_BF16) return run(__nv_bfloat16());
+    return MSPL_ERR_BAD_ARG;
 }
 
 template <int K, typename TT>

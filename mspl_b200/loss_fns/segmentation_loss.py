@@ -7,6 +7,12 @@ from torch import nn
 from .. import ops
 
 
+def _upcast(x):
+    """fp16 / bf16 (autocast) tensors as fp32, through a differentiable cast: autocast runs the reference's softmax and
+    log_softmax in fp32, so these modules compute in fp32 and hand the gradients back in the input's dtype."""
+    return x.float() if x.dtype in ops.HALF_DTYPES else x
+
+
 class PixelwiseKLD(nn.Module):
     """loss_fns/segmentation_loss.py:177-189: per-pixel KL(softmax(dist1) || softmax(dist2)), (B,C,H,W)x2 -> (B,H,W),
     differentiable w.r.t. both inputs."""
@@ -15,7 +21,7 @@ class PixelwiseKLD(nn.Module):
         super(PixelwiseKLD, self).__init__()
 
     def forward(self, dist1, dist2):
-        return ops.pixelwise_kld(dist1.contiguous(), dist2.contiguous())
+        return ops.pixelwise_kld(_upcast(dist1).contiguous(), _upcast(dist2).contiguous())
 
 
 class UncertaintyWeightedSegmentationLoss(nn.Module):
@@ -39,7 +45,7 @@ class UncertaintyWeightedSegmentationLoss(nn.Module):
         cw = self.class_weights
         if cw.dtype != torch.float32 or cw.device != pred.device:
             cw = cw.to(device=pred.device, dtype=torch.float32)
-        return ops.uw_segmentation_loss(pred.contiguous(), target.contiguous(), u_weight, cw.contiguous())
+        return ops.uw_segmentation_loss(_upcast(pred).contiguous(), target.contiguous(), _upcast(u_weight), cw.contiguous())
 
 
 class FusedUncertaintyWeightedLoss(nn.Module):

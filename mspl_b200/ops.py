@@ -415,13 +415,23 @@ def _class_index_target(target):
     return _require_cuda(target, "target", torch.int64, 3), False
 
 
-def uw_ce_fwd_bwd(main, aux, target, class_weights, alpha=20.0, norm_pixels=None, grad_scale=1.0, backward=True, iou_counts=None):
+# fp16 / bf16 logits of K4 (mspl_uw_ce_step_half): torch dtype -> MSPL_DTYPE_F16 / MSPL_DTYPE_BF16
+HALF_DTYPES = {torch.float16: 1, torch.bfloat16: 2}
+
+
+def uw_ce_fwd_bwd(main, aux, target, class_weights, alpha=20.0, norm_pixels=None, grad_scale=1.0, backward=True, iou_counts=None,
+                  grad_scale_dev=None):
     """K4, explicit form: returns (out3, d_main, d_aux) with out3 = [loss, mean w*ce*exp(-kld), mean kld] on device and
     the gradients of loss*grad_scale (None, None when backward=False).  target: (N,H,W) class indices, int64 or uint8.
     iou_counts: optional (3, K) int64 CUDA tensor that the same launch ADDS the MIOU.get_iou(main, target) pixel counts to
-    ([intersection | prediction | mask] per class, utilities/metrics/segmentation_miou.py:13-44 with num_classes = K)."""
-    main = _require_cuda(main, "main", torch.float32, 4)
-    aux = _require_cuda(aux, "aux", torch.float32, 4)
+    ([intersection | prediction | mask] per class, utilities/metrics/segmentation_miou.py:13-44 with num_classes = K).
+
+    main/aux may also both be fp16 or both bf16 (autocast logits): the kernel upcasts them exactly and computes in fp32, out3
+    stays fp32 and the gradients come back in the logits' dtype, scaled by grad_scale (and, for these dtypes only, by the
+    device scalar grad_scale_dev, a 1-element fp32 tensor) before they are rounded."""
+    half = isinstance(main, torch.Tensor) and main.dtype in HALF_DTYPES
+    main = _require_cuda(main, "main", main.dtype if half else torch.float32, 4)
+    aux = _require_cuda(aux, "aux", main.dtype, 4)
     target, u8 = _class_index_target(target)
     cw = _require_cuda(class_weights, "class_weights", torch.float32, 1)
     n, k, h, w = main.shape
@@ -431,6 +441,12 @@ def uw_ce_fwd_bwd(main, aux, target, class_weights, alpha=20.0, norm_pixels=None
     if k > MAX_CLASSES:
         raise NotImplementedError("fused loss supports up to %d classes; use PixelwiseKLD + "
                                   "UncertaintyWeightedSegmentationLoss modules for %d" % (MAX_CLASSES, k))
+    if grad_scale_dev is not None:
+        if not half:
+            raise ValueError("grad_scale_dev applies to fp16 / bf16 logits; scale fp32 gradients with grad_scale")
+        _require_cuda(grad_scale_dev, "grad_scale_dev", torch.float32)
+        if grad_scale_dev.numel() != 1:
+            raise ValueError("grad_scale_dev must hold one value")
     dev = main.device
     out3 = torch.empty(3, dtype=torch.float32, device=dev)
     d_main = torch.empty_like(main) if backward else None
@@ -442,10 +458,15 @@ def uw_ce_fwd_bwd(main, aux, target, class_weights, alpha=20.0, norm_pixels=None
         if iou_counts.shape != (3, k) or iou_counts.device != dev:
             raise ValueError("iou_counts must be a (3, %d) int64 tensor on %s" % (k, dev))
     with torch.cuda.device(dev):
-        st = _lib.load().mspl_uw_ce_step(_ptr(main), _ptr(aux), _ptr(target), int(u8), _ptr(cw), n, k, h * w, float(alpha), norm,
-                                         float(grad_scale), _ptr(out3), _ptr(d_main), _ptr(d_aux), _ptr(iou_counts), _ptr(ws),
-                                         ws.numel(), _stream(dev))
-    _lib.check(st, "mspl_uw_ce_step")
+        if half:
+            st = _lib.load().mspl_uw_ce_step_half(_ptr(main), _ptr(aux), HALF_DTYPES[main.dtype], _ptr(target), int(u8), _ptr(cw), n,
+                                                  k, h * w, float(alpha), norm, float(grad_scale), _ptr(grad_scale_dev), _ptr(out3),
+                                                  _ptr(d_main), _ptr(d_aux), _ptr(iou_counts), _ptr(ws), ws.numel(), _stream(dev))
+        else:
+            st = _lib.load().mspl_uw_ce_step(_ptr(main), _ptr(aux), _ptr(target), int(u8), _ptr(cw), n, k, h * w, float(alpha), norm,
+                                             float(grad_scale), _ptr(out3), _ptr(d_main), _ptr(d_aux), _ptr(iou_counts), _ptr(ws),
+                                             ws.numel(), _stream(dev))
+    _lib.check(st, "mspl_uw_ce_step_half" if half else "mspl_uw_ce_step")
     return out3, d_main, d_aux
 
 
@@ -453,14 +474,30 @@ class _UwCeLoss(torch.autograd.Function):
     @staticmethod
     def forward(ctx, main, aux, target, class_weights, alpha, norm_pixels, iou_counts=None):
         need = main.requires_grad or aux.requires_grad
-        out3, d_main, d_aux = uw_ce_fwd_bwd(main.detach(), aux.detach(), target, class_weights.detach(), alpha, norm_pixels,
-                                            1.0, backward=need, iou_counts=iou_counts)
-        ctx.grads = (d_main, d_aux)
+        ctx.deferred = main.dtype in HALF_DTYPES and need
+        if ctx.deferred:
+            # fp16 / bf16: the gradients must be scaled by the upstream gradient (a GradScaler's loss scale) before they are
+            # rounded, and that scale is only known in backward.  So this launch is forward-only, and backward runs K4 once more
+            # with the upstream gradient as its device scale.
+            out3, _, _ = uw_ce_fwd_bwd(main.detach(), aux.detach(), target, class_weights.detach(), alpha, norm_pixels,
+                                       backward=False, iou_counts=iou_counts)
+            ctx.save_for_backward(main, aux, target, class_weights)
+            ctx.cfg = (alpha, norm_pixels)
+            ctx.grads = None
+        else:
+            out3, d_main, d_aux = uw_ce_fwd_bwd(main.detach(), aux.detach(), target, class_weights.detach(), alpha, norm_pixels,
+                                                1.0, backward=need, iou_counts=iou_counts)
+            ctx.grads = (d_main, d_aux)
         ctx.mark_non_differentiable(out3)
         return out3[0].clone(), out3
 
     @staticmethod
     def backward(ctx, grad_loss, _grad_parts):
+        if getattr(ctx, "deferred", False):
+            main, aux, target, cw = ctx.saved_tensors
+            g = grad_loss.detach().to(torch.float32).reshape(1).contiguous()
+            _, d_main, d_aux = uw_ce_fwd_bwd(main.detach(), aux.detach(), target, cw.detach(), *ctx.cfg, grad_scale_dev=g)
+            return d_main, d_aux, None, None, None, None, None
         if ctx.grads is None:
             raise RuntimeError("uw_ce_loss: backward through this loss a second time is not supported (its gradients are "
                                "produced by the forward launch and handed over once)")
@@ -482,7 +519,9 @@ def uw_ce_loss(main, aux, target, class_weights, alpha=20.0, norm_pixels=None, r
     """K4 with autograd: the value of ``criterion(main + 0.5*aux, target, kld) * alpha + kld.mean()`` with
     ``kld = PixelwiseKLD()(main, aux)`` (uest_seg_multi_os.py:1020-1023), forward and backward in ONE kernel launch.
     norm_pixels overrides the divisor of the means (global pixel count under data parallelism); iou_counts: see
-    uw_ce_fwd_bwd (the training loop's ``miou_class.get_iou(pred, labels)`` of :1032 counted by the same launch)."""
+    uw_ce_fwd_bwd (the training loop's ``miou_class.get_iou(pred, labels)`` of :1032 counted by the same launch).
+    fp16 / bf16 logits (autocast) take one forward-only launch here and one forward+backward launch in backward, which scales
+    the gradients by the upstream gradient before rounding them to the logits' dtype."""
     loss, parts = _UwCeLoss.apply(main, aux, target, class_weights, alpha, norm_pixels, iou_counts)
     return (loss, parts) if return_parts else loss
 
